@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: Gk-mers/s counted for a K=25 spectrum (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (extract -> canonicalise -> partition -> sort -> count ->
-spectrum + sorted (k-mer, count) table) over the whole synthetic read set.
+spectrum + sorted (k-mer, count) table) over the whole synthetic read set.  --steps K timed steps follow the
+warm-up; --dump-outputs DIR writes what the last of them computed as float64 .npy files (see dump_outputs).
 
 Workload (config.workload): BASELINE.json configs[2], the largest single-GPU configuration --
 synthetic 100 Mb genome, 60 M x 100 bp reads (60x), K=25, 4.56 G k-mer instances per GPU.
@@ -259,6 +260,45 @@ def sampled_parity(kc, host, n_reads):
             "windows_scanned": int(n_win), "seconds": round(time.perf_counter() - t0, 2)}
 
 
+DUMP_BLOCKS, DUMP_BLOCK_ROWS, DUMP_SEED = 256, 2048, 2025   # table sample: 256 blocks of 2048 consecutive rows
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, kc, spec, n_instances, n_distinct):
+    """What a caller of the timed path receives, as float64 .npy files in out_dir, so that two builds can be compared
+    output for output on the same seeded reads:
+      spectrum.npy      dense spectrum, index = frequency
+      totals.npy        [k-mer instances, distinct k-mers]
+      table_rows.npy    row numbers of the sampled records of the sorted (k-mer, count) table
+      table_kmers.npy   their k-mers (one word each: 2K = 50 bits, exact in float64)
+      table_counts.npy  their counts
+    The table (617 M records at the default size) is sampled: DUMP_BLOCKS runs of DUMP_BLOCK_ROWS consecutive rows at
+    seeded offsets, one run per equal slice of the table; a table of at most that many rows is written whole.
+    With several ranks, the spectrum and totals are global and the table is this rank's shard."""
+    assert 2 * K <= 53 and kc.W == 1
+    n_rows = kc.totals()[1]
+    if n_rows <= DUMP_BLOCKS * DUMP_BLOCK_ROWS:
+        starts, size = [0], n_rows
+    else:
+        rng = np.random.default_rng(DUMP_SEED)
+        edges = [n_rows * b // DUMP_BLOCKS for b in range(DUMP_BLOCKS + 1)]
+        starts = [lo + int(rng.integers(0, hi - lo - DUMP_BLOCK_ROWS + 1)) for lo, hi in zip(edges, edges[1:])]
+        size = DUMP_BLOCK_ROWS
+    rows, kmers, counts = [], [], []
+    for first in starts:
+        k, c = kc.counts(first, size)
+        rows.append(np.arange(first, first + size, dtype=np.float64))
+        kmers.append(k[:, 0].astype(np.float64))
+        counts.append(c.astype(np.float64))
+    out = {"spectrum": np.asarray(spec, dtype=np.float64), "totals": np.array([n_instances, n_distinct], dtype=np.float64),
+           "table_rows": np.concatenate(rows), "table_kmers": np.concatenate(kmers), "table_counts": np.concatenate(counts)}
+    if sum(a.nbytes for a in out.values()) > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: the outputs exceed %d bytes" % DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
 
@@ -354,6 +394,11 @@ def run_ours(args):
     stage_ms = {k_: v / args.steps for k_, v in stage_acc.items()}
     geo = kc.geometry()
     n_local, nd_local = kc.totals()
+    if args.dump_outputs and rank == 0:   # before the e2e region below recounts the same reads
+        if world == 1:
+            dump_outputs(args.dump_outputs, kc, kc.spectrum(), n_local, nd_local)
+        else:
+            dump_outputs(args.dump_outputs, kc, kc._group.spectrum(), *kc._group.totals())
 
     # ---------------- e2e: host buffers through the public API, H2D + D2H inside the timed region
     nbytes = ((total_bases + 31) // 32) * 8
@@ -376,7 +421,7 @@ def run_ours(args):
     step_e2e()
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(1, args.steps)
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         spec = step_e2e()
     barrier()
@@ -533,7 +578,13 @@ def main():
     ap.add_argument("--workload", default="celegans", choices=["celegans", "human"],
                     help="celegans: BASELINE configs[2] per GPU (weak scaling, the default); human: configs[3], the 3 Gb x 45x "
                          "read set split over the GPUs (k-mer-space rounds; meant for --gpus 8)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float64; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.workload == "human":
         global READS_PER_GPU, GENOME_PER_GPU, CPU_SAMPLE_GENOME, WORKLOAD
         world = max(1, int(os.environ.get("WORLD_SIZE", args.gpus)))

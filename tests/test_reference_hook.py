@@ -1,24 +1,35 @@
-"""The hook that pins parity the day the reference source is mounted: `make -C oracle _ref` compiles the reference's own
-k-mer layer from /root/reference (never copied into this repo).  With the empty mount of rounds 1-2 the target is a
-no-op and the pinning test skips -- the oracle stays a spec-derived restatement ("parity unpinned", SURVEY.md 8c)."""
-import glob
+"""The hook that pins parity the day the reference source is available: `make -C oracle _ref REF=<dir>` compiles the
+reference's own k-mer layer from <dir>/src/kmers (never copied into this repo).  Without those sources the target is
+a no-op and the pinning test skips -- the oracle stays a spec-derived restatement ("parity unpinned", SURVEY.md 8c)."""
 import os
+import shutil
 import subprocess
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
-def test_ref_target_runs_and_reports():
-    out = subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "_ref"], capture_output=True, text=True)
-    assert out.returncode == 0, out.stderr
-    have_src = bool(glob.glob(os.path.join(REF, "src", "kmers", "KmerSpectra.cc")))
-    if have_src:
-        assert os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_kmers.so")), out.stdout
-    else:
-        assert "parity unpinned" in out.stdout
+def test_ref_target_runs_and_reports(tmp_path):
+    """`make _ref` on a copy of oracle/Makefile (so nothing lands in this tree): a reference directory without k-mer
+    sources builds nothing and says so; with them (a stand-in source here) the library is compiled."""
+    mk = tmp_path / "oracle"
+    mk.mkdir()
+    shutil.copy(os.path.join(ROOT, "oracle", "Makefile"), str(mk))
+    src = tmp_path / "reference" / "src" / "kmers"
+    src.mkdir(parents=True)
+
+    def make_ref():
+        out = subprocess.run(["make", "-C", str(mk), "-s", "_ref", "REF=%s" % (tmp_path / "reference")],
+                             capture_output=True, text=True)
+        assert out.returncode == 0, out.stderr
+        return out.stdout
+
+    assert "parity unpinned" in make_ref()
+    assert not (mk / "_ref").exists()
+    (src / "KmerSpectra.cc").write_text("int kmer_spectra_stand_in() { return 0; }\n")
+    stdout = make_ref()
+    assert (mk / "_ref" / "libref_kmers.so").exists(), stdout
 
 
 def test_oracle_against_the_reference_build():
