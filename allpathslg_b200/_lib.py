@@ -28,6 +28,11 @@ class GroupStats(C.Structure):
                 ("remote_bytes", C.c_uint64), ("gather_ms", C.c_float), ("step_ms", C.c_float)]
 
 
+class GroupFreqStats(C.Structure):
+    _fields_ = [("n_batches", C.c_int32), ("n_queries", C.c_uint64), ("remote_bytes", C.c_uint64), ("sweep_ms", C.c_float),
+                ("exchange_ms", C.c_float), ("scatter_ms", C.c_float), ("total_ms", C.c_float)]
+
+
 class SynthParams(C.Structure):
     _fields_ = [("genome_len", C.c_uint64), ("seed_g", C.c_uint64), ("seed_p", C.c_uint64), ("seed_q", C.c_uint64),
                 ("seed_r", C.c_uint64), ("seed_e", C.c_uint64), ("read_len", C.c_uint32), ("err_per_200", C.c_uint32)]
@@ -91,6 +96,7 @@ SYMBOLS = {
     "apgk_group_totals": (C.c_int, [_vp, _u64p, _u64p]),
     "apgk_group_spectrum_sparse": (C.c_int, [_vp, C.POINTER(_u64p), C.POINTER(_u64p), _u64p]),
     "apgk_group_stats_get": (C.c_int, [_vp, C.POINTER(GroupStats)]),
+    "apgk_group_read_freqs_device": (C.c_int, [_vp, _vp, _vp, _vp, C.POINTER(GroupFreqStats)]),
     "apgk_spectrum_device": (C.c_int, [_vp, C.POINTER(_vp), _u64p]),
     "apgk_spectrum_reload": (C.c_int, [_vp]),
     "apgk_stage_ms": (C.c_int, [_vp, C.POINTER(C.c_float)]),

@@ -19,7 +19,7 @@
 #include <vector>
 
 #include "../../include/apgk.h"
-#include "occ.cuh"
+#include "gfreq.cuh"
 
 using namespace apgk;
 
@@ -69,6 +69,7 @@ struct apgk_group;
 struct apgk_ctx {
   apgk_config cfg{};
   apgk_group* group = nullptr;       // the group this context is a member of (include/apgk.h "a GROUP of ranks")
+  uint64_t gen = 0;                  // bumped by every call that changes the read store or the table
   int W = 1;
   int device = 0;
   int n_sm = 148;
@@ -1249,8 +1250,9 @@ int occ_scatter_phase(apgk_ctx* c, unsigned long long* counters, OccScatter& o) 
   CU(cudaEventRecord(c->occ_ev[1], c->stream));
   constexpr int NT = 128;
   const uint64_t threads = (c->total_bases + POS_PER_THREAD - 1) / POS_PER_THREAD;
-  k_occ_scatter<W, Elem, NT><<<(unsigned)((threads + NT - 1) / NT), NT, 0, c->stream>>>(
-      read_store(c), freq_table<W>(c), c->occ_bcur.as<unsigned long long>(), (Elem*)o.elems, o.pos_tmp, o.pack_bits, N, counters);
+  k_occ_scatter<W, Elem, unsigned long long, NT><<<(unsigned)((threads + NT - 1) / NT), NT, 0, c->stream>>>(
+      read_store(c), freq_table<W>(c), 0, c->total_bases, nullptr, c->occ_bcur.as<unsigned long long>(), (Elem*)o.elems, o.pos_tmp,
+      o.pack_bits, N, counters);
   LAUNCHED();
   CU(cudaEventRecord(c->occ_ev[2], c->stream));
   return APGK_OK;
@@ -1700,6 +1702,7 @@ const char* apgk_last_error(const apgk_ctx* c) { return c ? c->err.c_str() : "nu
 
 int apgk_reset(apgk_ctx* c) {
   if (!c) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   { int rc = wait_ingest(c); if (rc) return rc; }
   if (c->total_bases) {
@@ -1714,6 +1717,7 @@ int apgk_reset(apgk_ctx* c) {
 
 int apgk_add_reads(apgk_ctx* c, const uint8_t* packed, const uint64_t* off, uint64_t n_reads) {
   if (!c || (!packed && n_reads) || (!off && n_reads)) return APGK_E_ARG;
+  c->gen++;
   if (!n_reads) return APGK_OK;
   CU(cudaSetDevice(c->device));
   { int rc = wait_ingest(c); if (rc) return rc; }
@@ -1743,6 +1747,7 @@ int apgk_add_reads(apgk_ctx* c, const uint8_t* packed, const uint64_t* off, uint
 
 int apgk_add_reads_uniform(apgk_ctx* c, const uint8_t* packed, uint64_t first_base, uint64_t n_reads, uint32_t read_len) {
   if (!c || (!packed && n_reads)) return APGK_E_ARG;
+  c->gen++;
   if (!n_reads || !read_len) return APGK_OK;
   CU(cudaSetDevice(c->device));
   const uint64_t nb = n_reads * (uint64_t)read_len;
@@ -1796,6 +1801,7 @@ int apgk_add_reads_uniform(apgk_ctx* c, const uint8_t* packed, uint64_t first_ba
 
 int apgk_synth_reads(apgk_ctx* c, const apgk_synth_params* p, uint64_t r0, uint64_t n_reads) {
   if (!c || !p) return APGK_E_ARG;
+  c->gen++;
   if (!n_reads) return APGK_OK;
   if (p->read_len == 0 || p->genome_len < p->read_len) FAIL(APGK_E_ARG, "genome shorter than a read");
   if (c->total_bases % 16) FAIL(APGK_E_STATE, "apgk_synth_reads needs the store to hold a multiple of 16 bases");
@@ -1838,6 +1844,7 @@ int apgk_read_store_info(const apgk_ctx* c, uint64_t* total_bases, uint64_t* n_r
 
 int apgk_finish(apgk_ctx* c) {
   if (!c) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   int rc = APGK_E_ARG;
   switch (c->W) {
@@ -1851,6 +1858,7 @@ int apgk_finish(apgk_ctx* c) {
 
 int apgk_finish_keys_device(apgk_ctx* c, const uint64_t* d_keys, uint64_t n) {
   if (!c || (!d_keys && n)) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   {  // the level-0 scatter writes c->A: keys handed in through apgk_key_buffer would be read and overwritten at once
     const unsigned char* k0 = (const unsigned char*)d_keys;
@@ -1887,6 +1895,7 @@ int apgk_choose_prefix_bits(apgk_ctx* c, uint64_t upper, int32_t* prefix_bits) {
 
 int apgk_partition(apgk_ctx* c, int32_t prefix_bits) {
   if (!c || prefix_bits < 0 || prefix_bits > 24) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   switch (c->W) {
     case 1: return finish_impl<1>(c, nullptr, 0, RUN_PARTITION, prefix_bits);
@@ -1945,6 +1954,7 @@ int apgk_partition_subsizes(apgk_ctx* c, int32_t split_bits, int32_t* effective_
 int apgk_count_pieces(apgk_ctx* c, const void* d_recv, uint32_t n_src, const uint32_t* d_sizes_all,
                       const uint64_t* seg_off, uint64_t bucket_lo, uint64_t bucket_hi, int32_t split_bits) {
   if (!c || !d_sizes_all || !seg_off || n_src == 0 || n_src > 1024) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   std::vector<const void*> bases(n_src, d_recv);
   switch (c->W) {
@@ -1987,6 +1997,7 @@ int apgk_count_pieces_peer(apgk_ctx* c, const void* const* d_src_base, uint32_t 
                            const uint64_t* src_off, uint64_t bucket_lo, uint64_t bucket_hi, int32_t split_bits,
                            const uint32_t* d_sub_sizes) {
   if (!c || !d_src_base || !d_sizes_all || !src_off || n_src == 0 || n_src > 1024) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   std::vector<const void*> bases(d_src_base, d_src_base + n_src);
   for (uint32_t s = 0; s < n_src; s++)
@@ -2074,6 +2085,7 @@ int apgk_release_temp(apgk_ctx* c) {
 
 int apgk_reserve_table(apgk_ctx* c, uint64_t n_records) {
   if (!c) return APGK_E_ARG;
+  c->gen++;
   CU(cudaSetDevice(c->device));
   CU(cudaStreamSynchronize(c->stream));
   const size_t kb = (size_t)c->W * 8;
@@ -2402,6 +2414,12 @@ const char* apgk_group_last_error(const apgk_group* g) { return g ? g->err.c_str
 int apgk_group_count(apgk_group* g) {
   if (!g) return APGK_E_ARG;
   return group_count(g);
+}
+
+int apgk_group_read_freqs_device(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base, const uint64_t* n_bases,
+                                 apgk_group_freq_stats* stats) {
+  if (!g) return APGK_E_ARG;
+  return group_read_freqs(g, d_out, first_base, n_bases, stats);
 }
 
 int apgk_group_totals(const apgk_group* g, uint64_t* n_instances, uint64_t* n_distinct) {

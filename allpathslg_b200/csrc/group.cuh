@@ -81,6 +81,9 @@ struct RankState {   // per LOCAL context
   uint32_t nb = 0, nbf = 0;
   uint64_t n_prev = 0, shard_n = 0, remote_bytes = 0;
   std::vector<uint64_t> tot0;                   // own level-0 totals (multi-round steps)
+  uint64_t gen_counted = 0;                     // the context's generation when the last count finished
+  DevBuf gpos, gcnt;                            // lookups: batch-relative position per slot of B; counters
+  cudaEvent_t gev[6]{};                         // lookups: stage boundaries of a batch, start and end of the call
 };
 
 }  // namespace
@@ -96,6 +99,10 @@ struct apgk_group {
   uint64_t n_instances = 0, n_distinct = 0;
   apgk_group_stats stats{};
   bool counted = false;
+  // who owns what after the last count: (bucket_lo, bucket_hi, owner) over the 2^P coarse buckets of every inner
+  // round; they tile [0, 2^P).  freq_ready: that count kept tables (APGK_WANT_COUNTS), lookups can be made.
+  std::vector<std::array<uint32_t, 3>> own_segs;
+  bool freq_ready = false;
   bool dead = false;   // a member context was destroyed: the group can only be destroyed
 };
 
@@ -321,8 +328,9 @@ void group_detach(apgk_group* g, apgk_ctx* c) {
       for (size_t s = 0; s < r.mapped.size(); s++)
         if (r.mapped[s]) { cudaIpcCloseMemHandle(r.peer_B[s]); cudaIpcCloseMemHandle(r.peer_sub[s]); r.mapped[s] = false; }
     DevBuf* all[] = {&r.sizes32, &r.sizes_all, &r.tot32, &r.E_tot, &r.cost32, &r.E_cost, &r.plan_dev, &r.ptrs_dev, &r.red_in, &r.red_out, &r.ovf_out,
-                     &r.ovf_all, &r.tot0_red, &r.meta_dev, &r.meta_all, &r.bar};
+                     &r.ovf_all, &r.tot0_red, &r.meta_dev, &r.meta_all, &r.bar, &r.gpos, &r.gcnt};
     for (DevBuf* b : all) b->release();
+    for (cudaEvent_t& e : r.gev) { if (e) cudaEventDestroy(e); e = nullptr; }
     if (r.host) cudaFreeHost(r.host);
     r.host = nullptr; r.host_words = 0;
     if (r.ev_a) cudaEventDestroy(r.ev_a);
@@ -526,6 +534,7 @@ int group_count_typed(apgk_group* g, const std::vector<GroupMeta>& meta, bool si
 
   // ---- the rounds
   bool first_exchange = true;
+  std::vector<std::array<uint32_t, 3>> segs;   // ownership of every inner round (host bookkeeping for the lookups)
   for (const GRound& R : rounds) {
     for (RankState& r : g->rs) {
       apgk_ctx* c = r.c;
@@ -601,6 +610,12 @@ int group_count_typed(apgk_group* g, const std::vector<GroupMeta>& meta, bool si
         lo = std::max<uint32_t>(lo, (uint32_t)s_lo * (uint32_t)bins1);
         hi = std::min<uint32_t>(hi, (uint32_t)s_hi * (uint32_t)bins1);
         if (hi < lo) hi = lo;
+        if (i == 0)   // the bounds are the same on every rank: every rank's clamped range of this inner round
+          for (int s = 0; s < world; s++) {
+            const uint32_t a = std::max<uint32_t>((uint32_t)r.host[hl.plan + s], (uint32_t)s_lo * (uint32_t)bins1);
+            const uint32_t b = std::min<uint32_t>((uint32_t)r.host[hl.plan + s + 1], (uint32_t)s_hi * (uint32_t)bins1);
+            if (b > a) segs.push_back({a, b, (uint32_t)s});
+          }
         // the gathered shard, the per-bucket records (over the dead level-0 keys when everything ran at once)
         GCU(c->C2.ensure(std::max<uint64_t>(Nr, 1) * sizeof(ElemB) + 16));
         Key<W>* tmp_keys;
@@ -744,6 +759,16 @@ int group_count_typed(apgk_group* g, const std::vector<GroupMeta>& meta, bool si
     g->stats.gather_ms = c->stage_ms[ST_OWNER];
     g->stats.step_ms = c->stage_ms[ST_TOTAL];
   }
+  std::sort(segs.begin(), segs.end());
+  uint32_t covered = 0;
+  for (const auto& sg : segs) {
+    if (sg[0] != covered) GFAIL(APGK_E_RANGE, "ownership segments do not tile the bucket space (gap or overlap at bucket %u)", covered);
+    covered = sg[1];
+  }
+  if (covered != nb) GFAIL(APGK_E_RANGE, "ownership segments end at bucket %u of %u", covered, nb);
+  g->own_segs = segs;
+  g->freq_ready = want_table != 0;
+  for (RankState& r : g->rs) r.gen_counted = r.c->gen;
   g->counted = true;
   return APGK_OK;
 }
@@ -823,6 +848,234 @@ int group_count(apgk_group* g) {
                          : group_count_typed<1, Key<1>>(g, meta, single, cap_outer, cap_inner, d2, budget, inner_bytes);
   if (W == 2) return group_count_typed<2, Key<2>>(g, meta, single, cap_outer, cap_inner, d2, budget, inner_bytes);
   return group_count_typed<3, Key<3>>(g, meta, single, cap_outer, cap_inner, d2, budget, inner_bytes);
+}
+
+// ---------------------------------------------------------------- frequency lookups on the sharded table
+// apgk_group_read_freqs_device; the kernels and the data flow are described in gfreq.cuh.
+
+struct FreqMeta {   // what every rank tells the others before a lookup (all-gathered, host side)
+  int32_t status, pad_;   // 0, or the error this rank met while preparing
+  uint64_t n_bases, batch_bases, cap_B, cap_sub, ptr_B, ptr_sub;
+};
+
+// Everything that can fail on one rank alone is decided here, before the call's first collective, and travels to
+// the others in FreqMeta::status: a rank that failed on its own between two collectives would leave the others
+// waiting in the next one.
+int gfreq_prepare(apgk_group* g, int i, uint32_t* const* d_out, const uint64_t* first_base, const uint64_t* n_bases, FreqMeta& m) {
+  RankState& r = g->rs[i];
+  apgk_ctx* c = r.c;
+  const int me = g->rank0 + i;
+  m = FreqMeta{};
+  m.cap_B = c->B.cap; m.cap_sub = c->sub_sizes.cap;
+  m.ptr_B = (uint64_t)(uintptr_t)c->B.p; m.ptr_sub = (uint64_t)(uintptr_t)c->sub_sizes.p;
+  if (!d_out || !first_base || !n_bases) GFAIL(APGK_E_ARG, "apgk_group_read_freqs_device: d_out, first_base and n_bases are required");
+  if (!g->counted || !g->freq_ready)
+    GFAIL(APGK_E_STATE, "apgk_group_read_freqs_device needs a completed apgk_group_count with APGK_WANT_COUNTS");
+  if (c->gen != r.gen_counted)
+    GFAIL(APGK_E_STATE, "rank %d: its context was reset, given reads or counted on its own since apgk_group_count: count again", me);
+  if (first_base[i] > c->total_bases || n_bases[i] > c->total_bases - first_base[i])
+    GFAIL(APGK_E_ARG, "rank %d: bases [%llu, +%llu) lie beyond its read store of %llu bases", me, (unsigned long long)first_base[i],
+          (unsigned long long)n_bases[i], (unsigned long long)c->total_bases);
+  if (n_bases[i] && !d_out[i]) GFAIL(APGK_E_ARG, "rank %d: no output buffer", me);
+  m.n_bases = n_bases[i];
+  GCU(cudaSetDevice(c->device));
+  // batch size from the budget of the count's temp buffers: per base at most one element in B and one position
+  uint64_t budget = c->budget_bytes;
+  if (const char* e = getenv("APGK_BUDGET_BYTES")) { if (atoll(e) > 0) budget = (uint64_t)atoll(e); }   // tests: a small device
+  const uint64_t eb = c->elem_bytes;
+  m.batch_bases = std::min<uint64_t>(std::max<uint64_t>(budget / (eb + 4), 4096), 1ull << 31) & ~15ull;
+  const uint64_t per = std::min(m.batch_bases, m.n_bases);
+  const uint32_t nb = r.nb;
+  const int world = g->world;
+  GCU(r.gpos.ensure(std::max<uint64_t>(per, 1) * 4));
+  GCU(r.gcnt.ensure(64));
+  GCU(c->piece_off.ensure((size_t)world * ((size_t)nb + 1) * 8));
+  GCU(r.sizes32.ensure((size_t)nb * 4));
+  GCU(r.sizes_all.ensure((size_t)world * nb * 4));
+  GCU(c->occ_bcur.ensure((size_t)nb * 8));
+  GCU(r.ptrs_dev.ensure(3 * (size_t)world * 8));
+  GCU(r.red_out.ensure(64));
+  GCU(c->blocksum.ensure((((size_t)nb + 1 + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * 8));   // what scan_u32 takes
+  for (cudaEvent_t& e : r.gev) if (!e) GCU(cudaEventCreate(&e));
+  // B grows later, in refresh_exports (peers may have it mapped): here only whether it can
+  const uint64_t need_B = per * eb + 16;
+  if (need_B > c->B.cap) {
+    size_t fr = 0, tot = 0;
+    GCU(cudaMemGetInfo(&fr, &tot));
+    if ((uint64_t)fr + c->B.cap < need_B + (64ull << 20))
+      GFAIL(APGK_E_NOMEM, "rank %d: the partition buffer needs %llu bytes, %llu free", me, (unsigned long long)need_B, (unsigned long long)fr);
+  }
+  return APGK_OK;
+}
+
+template <int W, typename Elem>
+int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base, const std::vector<FreqMeta>& meta,
+                           apgk_group_freq_stats* st) {
+  const int world = g->world, nl = g->n_local;
+  constexpr uint64_t eb = sizeof(Elem);
+  uint64_t BB = ~0ull, n_batches = 0;
+  for (int s = 0; s < world; s++) BB = std::min<uint64_t>(BB, meta[s].batch_bases);
+  for (int s = 0; s < world; s++) n_batches = std::max<uint64_t>(n_batches, (meta[s].n_bases + BB - 1) / BB);
+  // every rank's B large enough for one batch, re-exported where it grew (after apgk_release_temp too)
+  {
+    std::vector<GroupMeta> gm(world);
+    std::vector<uint64_t> need_B(world);
+    for (int s = 0; s < world; s++) {
+      gm[s] = GroupMeta{};
+      gm[s].cap_B = meta[s].cap_B; gm[s].cap_sub = meta[s].cap_sub; gm[s].ptr_B = meta[s].ptr_B; gm[s].ptr_sub = meta[s].ptr_sub;
+      need_B[s] = std::min(BB, meta[s].n_bases) * eb + 16;
+    }
+    int rc = refresh_exports(g, gm, need_B, 16);
+    if (rc) return rc;
+  }
+  RankState& r0 = g->rs[0];
+  apgk_ctx* c0 = r0.c;
+  for (RankState& r : g->rs) {
+    apgk_ctx* c = r.c;
+    GCU(cudaSetDevice(c->device));
+    { int rc = wait_ingest(c); if (rc) return rc; }
+    GCU(cudaMemcpyAsync(r.ptrs_dev.p, r.peer_B.data(), (size_t)world * 8, cudaMemcpyHostToDevice, c->stream));
+    GCU(cudaMemsetAsync(r.gcnt.p, 0, 64, c->stream));
+  }
+  GCU(cudaSetDevice(c0->device));
+  GCU(cudaEventRecord(r0.gev[4], c0->stream));
+  float ms[3] = {0, 0, 0};
+  auto collect = [&]() {   // stage times of the batch just run, first local context
+    cudaEventSynchronize(r0.gev[3]);
+    for (int k = 0; k < 3; k++) { float x = 0; if (cudaEventElapsedTime(&x, r0.gev[k], r0.gev[k + 1]) == cudaSuccess) ms[k] += x; }
+  };
+  constexpr int NT = 128;
+  for (uint64_t k = 0; k < n_batches; k++) {
+    if (k) collect();
+    // -- sender: histogram of the batch's windows by coarse bucket, bucket starts, elements into B
+    for (int i = 0; i < nl; i++) {
+      RankState& r = g->rs[i];
+      apgk_ctx* c = r.c;
+      const int me = g->rank0 + i;
+      GCU(cudaSetDevice(c->device));
+      if (i == 0) GCU(cudaEventRecord(r.gev[0], c->stream));
+      const uint32_t nb = r.nb;
+      const uint64_t n = meta[me].n_bases, b0 = std::min(k * BB, n), nbb = std::min(BB, n - b0), first = first_base[i] + b0;
+      FreqTable<W> tp{};   // the partition geometry: the sweep reads only the bucket digit's position
+      tp.prefix_pos = r.geom_part.REM; tp.prefix_len = r.geom_part.D0 + r.geom_part.D1; tp.pad = r.geom_part.pad;
+      unsigned long long* own = c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)nb + 1);
+      unsigned long long* cnt = r.gcnt.as<unsigned long long>();
+      const unsigned grid = (unsigned)((((first & 15) + nbb + POS_PER_THREAD - 1) / POS_PER_THREAD + NT - 1) / NT);
+      GCU(cudaMemsetAsync(r.sizes32.p, 0, (size_t)nb * 4, c->stream));
+      if (nbb) {
+        GCU(cudaMemsetAsync(d_out[i] + b0, 0xFF, nbb * 4, c->stream));
+        k_occ_scatter<W, Elem, uint32_t, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, r.sizes32.as<uint32_t>(), nullptr,
+                                                                        nullptr, nullptr, 0, 0, cnt);
+        c->launches++;
+        GCU(cudaGetLastError());
+      }
+      GCTX(c, scan_u32(c, r.sizes32.as<uint32_t>(), nb, own, nullptr));
+      if (nbb) {
+        GCU(cudaMemcpyAsync(c->occ_bcur.p, own, (size_t)nb * 8, cudaMemcpyDeviceToDevice, c->stream));
+        k_occ_scatter<W, Elem, uint32_t, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, nullptr, c->occ_bcur.as<unsigned long long>(),
+                                                                        c->B.as<Elem>(), r.gpos.as<uint32_t>(), 0, nbb, cnt);
+        c->launches++;
+        GCU(cudaGetLastError());
+      }
+      if (i == 0) GCU(cudaEventRecord(r.gev[1], c->stream));
+    }
+    // -- every rank learns every rank's bucket sizes (this also orders the owners' reads after the senders' sweeps)
+    { int rc = coll_allgather_dev(g, (size_t)g->rs[0].nb * 4, [&](int i) { return (const void*)g->rs[i].sizes32.p; },
+                                  [&](int i) { return (void*)g->rs[i].sizes_all.p; }); if (rc) return rc; }
+    // -- owner: the pieces of its buckets, resolved in place in the senders' B
+    for (int i = 0; i < nl; i++) {
+      RankState& r = g->rs[i];
+      apgk_ctx* c = r.c;
+      const int me = g->rank0 + i;
+      const uint32_t nb = r.nb;
+      GCU(cudaSetDevice(c->device));
+      for (int s = 0; s < world; s++)
+        if (s != me)
+          GCTX(c, scan_u32(c, r.sizes_all.as<uint32_t>() + (size_t)s * nb, nb, c->piece_off.as<unsigned long long>() + (size_t)s * ((size_t)nb + 1), nullptr));
+      FreqTable<W> ts = freq_table<W>(c);   // the shard's table, indexed by the finer bucket of the count (P + d2 bits)
+      ts.nb = r.nbf; ts.prefix_pos = r.geom_shard.REM; ts.prefix_len = r.geom_shard.D0 + r.geom_shard.D1; ts.pad = r.geom_shard.pad;
+      ts.D1 = r.geom_shard.D1;
+      GfArgs<Elem> a{};
+      a.src = (Elem* const*)r.ptrs_dev.p; a.piece_off = c->piece_off.as<unsigned long long>();
+      a.n_src = (uint32_t)world; a.nb = nb; a.me = (uint32_t)me;
+      a.d2 = r.geom_shard.D1 - r.geom_part.D1; a.rem_bits = r.geom_part.REM; a.pad = r.geom_part.pad;
+      a.counters = r.gcnt.as<unsigned long long>();
+      for (const auto& sg : g->own_segs) {
+        if ((int)sg[2] != me) continue;
+        a.lo = sg[0]; a.hi = sg[1];
+        k_gf_resolve<W, Elem, GF_NT><<<std::min<uint32_t>(sg[1] - sg[0], (uint32_t)c->n_sm * 8), GF_NT, 0, c->stream>>>(ts, a);
+        c->launches++;
+        GCU(cudaGetLastError());
+      }
+    }
+    // -- all owners are done.  Their stores into this rank's B were made by kernels that had completed when their
+    // streams reached the barrier; a kernel's stores, peer stores included, are visible to every device once it has
+    // completed, and this rank's scatter runs after the barrier on its stream.  (The barrier also keeps the next
+    // batch's sweep from overwriting B while an owner still reads it.)
+    { int rc = coll_barrier_dev(g); if (rc) return rc; }
+    for (int i = 0; i < nl; i++) {
+      RankState& r = g->rs[i];
+      apgk_ctx* c = r.c;
+      const int me = g->rank0 + i;
+      GCU(cudaSetDevice(c->device));
+      if (i == 0) GCU(cudaEventRecord(r.gev[2], c->stream));
+      const uint64_t n = meta[me].n_bases, b0 = std::min(k * BB, n), nbb = std::min(BB, n - b0);
+      if (nbb) {
+        const unsigned long long* own = c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)r.nb + 1);
+        k_gf_scatter<Elem><<<(unsigned)std::min<uint64_t>((nbb + 255) / 256, (uint64_t)c->n_sm * 8), 256, 0, c->stream>>>(
+            c->B.as<Elem>(), r.gpos.as<uint32_t>(), own + r.nb, d_out[i] + b0, r.gcnt.as<unsigned long long>());
+        c->launches++;
+        GCU(cudaGetLastError());
+      }
+      if (i == 0) GCU(cudaEventRecord(r.gev[3], c->stream));
+    }
+  }
+  // windows missing from their owner's table (or beyond their bucket) summed over the ranks: a table that does not
+  // match the reads fails the call on every rank
+  { int rc = coll_allreduce_u64(g, 4, false, [&](int i) { return (const void*)g->rs[i].gcnt.p; },
+                                [&](int i) { return (void*)g->rs[i].red_out.p; }); if (rc) return rc; }
+  unsigned long long red[4] = {0, 0, 0, 0}, own[4] = {0, 0, 0, 0};
+  GCU(cudaSetDevice(c0->device));
+  GCU(cudaEventRecord(r0.gev[5], c0->stream));
+  GCU(cudaMemcpyAsync(red, r0.red_out.p, 32, cudaMemcpyDeviceToHost, c0->stream));
+  GCU(cudaMemcpyAsync(own, r0.gcnt.p, 32, cudaMemcpyDeviceToHost, c0->stream));
+  for (RankState& r : g->rs) { GCU(cudaSetDevice(r.c->device)); GCU(cudaStreamSynchronize(r.c->stream)); }
+  if (n_batches) collect();
+  if (red[0] || red[2])
+    GFAIL(APGK_E_STATE, "group read_freqs: %llu windows missing from their owner's table, %llu beyond their bucket (the tables do not match the reads)",
+          red[0], red[2]);
+  if (st) {
+    *st = apgk_group_freq_stats{};
+    st->n_batches = (int32_t)n_batches;
+    st->n_queries = own[3];
+    st->remote_bytes = own[1] * (eb + 4);
+    st->sweep_ms = ms[0]; st->exchange_ms = ms[1]; st->scatter_ms = ms[2];
+    cudaEventElapsedTime(&st->total_ms, r0.gev[4], r0.gev[5]);
+  }
+  return APGK_OK;
+}
+
+int group_read_freqs(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base, const uint64_t* n_bases, apgk_group_freq_stats* st) {
+  if (g->dead) GFAIL(APGK_E_STATE, "a context of this group has been destroyed");
+  const int world = g->world, nl = g->n_local;
+  std::vector<FreqMeta> mine(nl), meta(world);
+  std::string own_err;
+  for (int i = 0; i < nl; i++) {
+    const int rc = gfreq_prepare(g, i, d_out, first_base, n_bases, mine[i]);
+    if (rc) { mine[i].status = rc; if (own_err.empty()) own_err = g->err; }
+  }
+  { int rc = coll_allgather_host(g, mine.data(), sizeof(FreqMeta), meta.data()); if (rc) return rc; }
+  for (int s = 0; s < world; s++)
+    if (meta[s].status) {
+      if (own_err.empty()) GFAIL(meta[s].status, "rank %d refused the lookup (error %d; its apgk_group_last_error says why)", s, meta[s].status);
+      g->err = own_err;
+      return meta[s].status;
+    }
+  apgk_ctx* c0 = g->rs[0].c;
+  if (c0->elem_bytes == 4) return group_read_freqs_typed<1, uint32_t>(g, d_out, first_base, meta, st);
+  if (c0->W == 1) return group_read_freqs_typed<1, Key<1>>(g, d_out, first_base, meta, st);
+  if (c0->W == 2) return group_read_freqs_typed<2, Key<2>>(g, d_out, first_base, meta, st);
+  return group_read_freqs_typed<3, Key<3>>(g, d_out, first_base, meta, st);
 }
 
 }  // namespace

@@ -95,24 +95,36 @@ __global__ void k_occ_bstart(const unsigned long long* __restrict__ index, const
 // (32-bit remainders whose REM bits fit above the position in one word): pos_tmp[o] = rem << pack_bits | pos,
 // one 8-byte store per window; else the element and the position go to two arrays.  A slot can only run
 // past its bucket if the table does not match the read store; k_occ_place would then miss the k-mer.
-template <int W, typename Elem, int NT>
-__global__ void __launch_bounds__(NT) k_occ_scatter(ReadStore rs, FreqTable<W> t, unsigned long long* __restrict__ bcur,
-                                                    Elem* __restrict__ elems, unsigned long long* __restrict__ pos_tmp,
+// Only the windows starting in [first, first + n_bases) take part (the whole store for the single-GPU forms).
+// Pos = unsigned long long: pos = (global base position << 1) | canonical-is-reverse; Pos = uint32_t: pos = base
+// position - first, never packed (the batches of the group lookups, csrc/gfreq.cuh).  hist != nullptr: the
+// sweep only counts the windows of every bucket into hist[b] and places nothing.
+template <int W, typename Elem, typename Pos, int NT>
+__global__ void __launch_bounds__(NT) k_occ_scatter(ReadStore rs, FreqTable<W> t, uint64_t first, uint64_t n_bases,
+                                                    uint32_t* __restrict__ hist, unsigned long long* __restrict__ bcur,
+                                                    Elem* __restrict__ elems, Pos* __restrict__ pos_tmp,
                                                     int pack_bits, unsigned long long n_slots,
                                                     unsigned long long* __restrict__ counters) {
-  const uint64_t p = ((uint64_t)blockIdx.x * NT + threadIdx.x) * POS_PER_THREAD;
-  if (p >= rs.total_bases) return;
-  const uint32_t valid = window_valid_mask16(rs.starts32, p, rs.K, rs.total_bases);
+  const uint64_t p = (first & ~15ull) + ((uint64_t)blockIdx.x * NT + threadIdx.x) * POS_PER_THREAD;
+  const uint64_t end = first + n_bases;
+  if (p >= end) return;
+  uint32_t valid = window_valid_mask16(rs.starts32, p, rs.K, rs.total_bases);
+  if (p < first) valid &= 0xFFFFu << (uint32_t)(first - p);
+  if (end - p < 16) valid &= (1u << (uint32_t)(end - p)) - 1u;
   if (!valid) return;
   Window16<W> win;
   load_window16<W>(rs.bases32, p, rs.K, win);
   extract16<W>(win, rs.K, [&](int j, const Key<W>& c, bool use_rc) {
     if ((valid >> j) & 1u) {
       const uint32_t b = digit_of(c, t.prefix_pos, t.prefix_len, t.pad);
+      if (hist) { atomicAdd(&hist[b], 1u); return; }
       const unsigned long long o = atomicAdd(&bcur[b], 1ull);   // (a 32-bit relative cursor + a read of bstart[b] measured 10 % slower)
       const unsigned long long pv = ((p + (uint64_t)j) << 1) | (use_rc ? 1ull : 0ull);
       if (o >= n_slots) {
         atomicAdd(&counters[2], 1ull);
+      } else if constexpr (sizeof(Pos) == 4) {
+        elems[o] = OccElem<Elem, W>::make(c, t.prefix_pos, t.pad);
+        pos_tmp[o] = (Pos)(p + (uint64_t)j - first);
       } else if constexpr (sizeof(Elem) == 4) {
         const uint32_t r = OccElem<Elem, W>::make(c, t.prefix_pos, t.pad);
         if (pack_bits) {

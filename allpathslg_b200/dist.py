@@ -87,6 +87,14 @@ def sharded_count(kc, rank, world, group=None, timings=None):
     return grp.spectrum(), ni, nd
 
 
+def sharded_read_freqs(kc, rank, world, first_base=0, n_bases=None, group=None, stats=None):
+    """After `sharded_count`: the GLOBAL count of the canonical k-mer at every base of [first_base, first_base +
+    n_bases) of this rank's read store (default: to its end), as a host uint32 array (0xFFFFFFFF where the window
+    leaves its read).  Collective: every rank calls it, each with its own range (apgk_group_read_freqs_device)."""
+    grp = _group_of(kc, rank, world, group)
+    return grp.read_freqs([first_base], None if n_bases is None else [n_bases], stats=stats)[0]
+
+
 def _group_of(kc, rank, world, group=None):
     """The library-side group of this counter (made once: rank 0's id is broadcast over torch.distributed)."""
     from .kmers import KmerGroup

@@ -49,6 +49,7 @@ class KmerCounter:
         self._L = _lib.lib()
         self.K = int(K)
         self.W = words_per_kmer(self.K)
+        self.device = int(device)
         cfg = Config(K=self.K, device=device,
                      flags=WANT_SPECTRUM | (WANT_COUNTS if want_counts else 0) | (ASYNC_INGEST if async_ingest else 0),
                      prefix_bits=prefix_bits, reserve_bases=reserve_bases, max_round_keys=max_round_keys,
@@ -422,6 +423,45 @@ class KmerGroup:
         st = _lib.GroupStats()
         self._ck(self._L.apgk_group_stats_get(self._h, C.byref(st)))
         return {k: getattr(st, k) for k, _ in st._fields_}
+
+    def read_freqs_device(self, d_outs, first_base=None, n_bases=None):
+        """Frequency lookups on the sharded table (collective): for every local counter j, d_outs[j] (a DEVICE pointer
+        on that counter's device, n_bases[j] uint32) receives the GLOBAL count of the canonical k-mer at every base of
+        [first_base[j], first_base[j] + n_bases[j]) of its read store, 0xFFFFFFFF where the window leaves its read.
+        Defaults: the whole store.  -> dict(n_batches, n_queries, remote_bytes, sweep_ms, exchange_ms, scatter_ms,
+        total_ms)."""
+        first_base, n_bases = self._ranges(first_base, n_bases)
+        n = len(self.counters)
+        outs = (C.c_void_p * n)(*[int(p) if p else None for p in d_outs])
+        fb = np.ascontiguousarray(first_base, dtype=np.uint64)
+        nb = np.ascontiguousarray(n_bases, dtype=np.uint64)
+        st = _lib.GroupFreqStats()
+        self._ck(self._L.apgk_group_read_freqs_device(self._h, outs, fb.ctypes.data, nb.ctypes.data, C.byref(st)))
+        return {k: getattr(st, k) for k, _ in st._fields_}
+
+    def read_freqs(self, first_base=None, n_bases=None, stats=None):
+        """The same into host arrays: a list of uint32 arrays, one per local counter (device buffers from torch on each
+        counter's device).  stats: a dict to receive the call's statistics."""
+        import torch
+
+        first_base, n_bases = self._ranges(first_base, n_bases)
+        bufs = [torch.empty(max(int(n), 1), dtype=torch.int32, device="cuda:%d" % kc.device)
+                for kc, n in zip(self.counters, n_bases)]
+        st = self.read_freqs_device([b.data_ptr() for b in bufs], first_base, n_bases)
+        if stats is not None:
+            stats.update(st)
+        return [b.cpu().numpy().view(np.uint32)[: int(n)] for b, n in zip(bufs, n_bases)]
+
+    def _ranges(self, first_base, n_bases):
+        n = len(self.counters)
+        if first_base is None:
+            first_base = [0] * n
+        if n_bases is None:
+            n_bases = [kc.read_store_info()[0] - int(f) for kc, f in zip(self.counters, first_base)]
+        first_base, n_bases = [int(x) for x in first_base], [int(x) for x in n_bases]
+        if len(first_base) != n or len(n_bases) != n:
+            raise ValueError("one first_base and one n_bases per local counter")
+        return first_base, n_bases
 
     def close(self):
         if getattr(self, "_h", None):

@@ -295,6 +295,29 @@ typedef struct {
   float step_ms;              /* device time of the whole call on that context's stream */
 } apgk_group_stats;
 int apgk_group_stats_get(const apgk_group* g, apgk_group_stats* out);
+/* Frequency lookups on the sharded table: the bulk form of apgk_read_freqs for a group.  Each rank's reads contain
+ * k-mers every rank owns, so the queries travel to their owner: per batch of the base range, every rank sends its
+ * windows' level-1 elements (4-byte remainder or full key) bucket by bucket through its partition buffer, each owner
+ * resolves the pieces of the buckets it owns against its table over peer memory and writes the counts back in place,
+ * and every rank scatters the answers to the positions.  Batches are sized from the device-memory budget of the
+ * count; every rank runs the same number of them.
+ * After apgk_group_count with APGK_WANT_COUNTS: for every base i of [first_base[j], first_base[j] + n_bases[j]) of the
+ * read store of the group's j-th LOCAL context, d_out[j][i - first_base[j]] = the GLOBAL count of the canonical k-mer
+ * starting there (0xFFFFFFFF where the window leaves its read).  This is what apgk_read_freqs_device gives on one GPU,
+ * with the counts held by the shards.  Collective.  Arrays have one entry per local context (one in the multi-process
+ * form).  d_out: DEVICE buffers of n_bases[j] uint32 on that context's device (NULL allowed where n_bases[j] == 0).
+ * stats may be NULL.  Errors are decided from values all ranks share and come back identical on every rank:
+ * APGK_E_STATE without a current count with APGK_WANT_COUNTS, or when a member context was reset, given reads or
+ * counted on its own since (apgk_release_temp is fine), or when a window's k-mer is missing from its owner's table;
+ * APGK_E_ARG for a range beyond a read store or a missing buffer; APGK_E_NOMEM when a rank's buffers do not fit. */
+typedef struct {
+  int32_t n_batches;        /* exchange batches this call ran (agreed by all ranks) */
+  uint64_t n_queries;       /* valid windows of this rank's range that were resolved */
+  uint64_t remote_bytes;    /* bytes this rank's owner-side kernels read from and wrote to peers' memory */
+  float sweep_ms, exchange_ms, scatter_ms, total_ms;   /* device time, first local context */
+} apgk_group_freq_stats;
+int apgk_group_read_freqs_device(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base,
+                                 const uint64_t* n_bases, apgk_group_freq_stats* stats);
 
 /* ---- instrumentation */
 #define APGK_N_STAGES 14
