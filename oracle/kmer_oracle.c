@@ -333,11 +333,17 @@ int oracle_count(const uint8_t* packed, const uint64_t* off, uint64_t n_reads, i
  * with the device's table for the same key ranges.
  *
  * oracle_sample_prefix: the selected instances, unsorted (malloc'd, n * W words).  Reads are off[] delimited, or
- * uniform (off == NULL: n_reads reads of read_len bases back to back).  n_windows_out = ALL windows seen. */
-int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_reads, uint32_t read_len, int K, int pbits,
-                         const uint8_t* sel, int n_threads, uint64_t** keys_out, uint64_t* n_out, uint64_t* n_windows_out) {
+ * uniform (off == NULL: n_reads reads of read_len bases back to back).  n_windows_out = ALL windows seen.
+ * oracle_sample_prefix_pos: the same instances, plus one word per instance (malloc'd, n words):
+ * (q << 1) | canonical_is_reverse, q = the window's first base in the packed stream (off[] counts in it), reverse
+ * when the canonical form is the reverse complement of the window (a palindrome counts as forward).  Reads are
+ * split into equal slices in order and the slices concatenated in order, so the instances come ascending by q. */
+static int sample_prefix_impl(const uint8_t* packed, const uint64_t* off, uint64_t n_reads, uint32_t read_len, int K,
+                              int pbits, const uint8_t* sel, int n_threads, uint64_t** keys_out, uint64_t** pos_out,
+                              uint64_t* n_out, uint64_t* n_windows_out) {
   if (K < 1 || K > 32 * MAXW || pbits < 0 || pbits > 16 || pbits > 2 * K) return -1;
   int W = (2 * K + 63) / 64;
+  const int want_pos = pos_out != NULL;
 #ifdef _OPENMP
   if (n_threads <= 0) n_threads = omp_get_max_threads();
 #else
@@ -350,7 +356,8 @@ int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_
   uint64_t* cnt = (uint64_t*)calloc((size_t)T + 1, 8);
   uint64_t* win = (uint64_t*)calloc((size_t)T + 1, 8);
   uint64_t** bufs = (uint64_t**)calloc((size_t)T, sizeof(uint64_t*));
-  if (!cnt || !win || !bufs) return -2;
+  uint64_t** pbufs = (uint64_t**)calloc((size_t)T, sizeof(uint64_t*));
+  if (!cnt || !win || !bufs || !pbufs) return -2;
   int failed = 0;
 #pragma omp parallel num_threads(T)
   {
@@ -363,7 +370,8 @@ int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_
     uint64_t r_hi = n_reads / T * (t + 1) + (n_reads % T < (uint64_t)(t + 1) ? n_reads % T : (uint64_t)(t + 1));
     uint64_t n = 0, nw = 0, cap = 1u << 16;
     uint64_t* out = (uint64_t*)malloc(cap * (size_t)W * 8);   /* grows: the thread's selected instances */
-    int bad = out == NULL;
+    uint64_t* pout = want_pos ? (uint64_t*)malloc(cap * 8) : NULL;
+    int bad = out == NULL || (want_pos && pout == NULL);
     for (uint64_t r = r_lo; r < r_hi && !bad; r++) {
       uint64_t b0 = off ? off[r] : r * (uint64_t)read_len, b1 = off ? off[r + 1] : b0 + read_len;
       if (b1 - b0 < (uint64_t)K) continue;
@@ -372,6 +380,11 @@ int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_
         uint64_t* nb = (uint64_t*)realloc(out, cap * (size_t)W * 8);
         if (!nb) { bad = 1; break; }
         out = nb;
+        if (want_pos) {
+          uint64_t* np_ = (uint64_t*)realloc(pout, cap * 8);
+          if (!np_) { bad = 1; break; }
+          pout = np_;
+        }
       }
       if (W == 1) {
         uint64_t fw = 0, rc = 0, filled = 0;
@@ -383,6 +396,7 @@ int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_
             uint64_t c = fw < rc ? fw : rc;
             nw++;
             out[n] = c;
+            if (want_pos) pout[n] = ((q + 1 - (uint64_t)K) << 1) | (uint64_t)(rc < fw);
             n += sel[pbits ? (uint32_t)(c >> (topbits - pbits)) : 0] != 0;
           }
         }
@@ -394,10 +408,12 @@ int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_
           roll_fw(fw, W, topmask, b);
           roll_rc(rc, W, topshift, b);
           if (++filled >= (uint64_t)K) {
-            const uint64_t* c = cmp_w(fw, rc, W) <= 0 ? fw : rc;
+            int use_rc = cmp_w(rc, fw, W) < 0;
+            const uint64_t* c = use_rc ? rc : fw;
             nw++;
             if (sel[bucket_of(c, K, W, pbits)]) {
               for (int i = 0; i < W; i++) out[n * W + i] = c[i];
+              if (want_pos) pout[n] = ((q + 1 - (uint64_t)K) << 1) | (uint64_t)use_rc;
               n++;
             }
           }
@@ -408,22 +424,38 @@ int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_
 #pragma omp atomic write
       failed = 1;
     }
-    cnt[t + 1] = n; win[t] = nw; bufs[t] = out;
+    cnt[t + 1] = n; win[t] = nw; bufs[t] = out; pbufs[t] = pout;
   }
   for (int t = 0; t < T; t++) cnt[t + 1] += cnt[t];   /* cnt[t] = first output slot of thread t */
   uint64_t* keys = failed ? NULL : (uint64_t*)malloc((cnt[T] ? cnt[T] : 1) * (size_t)W * 8);
+  uint64_t* pos = failed || !want_pos ? NULL : (uint64_t*)malloc((cnt[T] ? cnt[T] : 1) * 8);
+  if (want_pos && !pos && keys) { free(keys); keys = NULL; }
   uint64_t nw = 0;
   for (int t = 0; t < T; t++) {
     if (keys && bufs[t]) memcpy(keys + cnt[t] * W, bufs[t], (cnt[t + 1] - cnt[t]) * (size_t)W * 8);
-    free(bufs[t]);
+    if (pos && pbufs[t]) memcpy(pos + cnt[t], pbufs[t], (cnt[t + 1] - cnt[t]) * 8);
+    free(bufs[t]); free(pbufs[t]);
     nw += win[t];
   }
   uint64_t n_all = cnt[T];
-  free(cnt); free(win); free(bufs);
+  free(cnt); free(win); free(bufs); free(pbufs);
   if (!keys) return -2;
   *keys_out = keys; *n_out = n_all;
+  if (want_pos) *pos_out = pos;
   if (n_windows_out) *n_windows_out = nw;
   return 0;
+}
+
+int oracle_sample_prefix(const uint8_t* packed, const uint64_t* off, uint64_t n_reads, uint32_t read_len, int K, int pbits,
+                         const uint8_t* sel, int n_threads, uint64_t** keys_out, uint64_t* n_out, uint64_t* n_windows_out) {
+  return sample_prefix_impl(packed, off, n_reads, read_len, K, pbits, sel, n_threads, keys_out, NULL, n_out, n_windows_out);
+}
+
+int oracle_sample_prefix_pos(const uint8_t* packed, const uint64_t* off, uint64_t n_reads, uint32_t read_len, int K,
+                             int pbits, const uint8_t* sel, int n_threads, uint64_t** keys_out, uint64_t** pos_out,
+                             uint64_t* n_out, uint64_t* n_windows_out) {
+  return sample_prefix_impl(packed, off, n_reads, read_len, K, pbits, sel, n_threads, keys_out, pos_out, n_out,
+                            n_windows_out);
 }
 
 /* oracle_count_keys: sort + count n canonical k-mer instances (W words each, any order; the array is consumed:

@@ -66,6 +66,9 @@ def lib():
         L.oracle_sample_prefix.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_int, C.c_int, C.c_void_p,
                                            C.c_int, C.POINTER(u64p), u64p, u64p]
         L.oracle_sample_prefix.restype = C.c_int
+        L.oracle_sample_prefix_pos.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_int, C.c_int,
+                                               C.c_void_p, C.c_int, C.POINTER(u64p), C.POINTER(u64p), u64p, u64p]
+        L.oracle_sample_prefix_pos.restype = C.c_int
         L.oracle_count_keys.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.POINTER(u64p), C.POINTER(u64p), u64p]
         L.oracle_count_keys.restype = C.c_int
         _lib = L
@@ -115,11 +118,7 @@ def count(packed, off, K, n_threads=0):
     return kmers, counts, ni.value
 
 
-def sample_prefix(packed, off, K, pbits, parts, n_reads=None, read_len=0, n_threads=0):
-    """Sampled-partition oracle, step 1 (SURVEY.md section 8c "human-scale check" ii): the canonical k-mer INSTANCES
-    of all reads whose leading `pbits` bits are one of `parts`.  packed: uint8 array or an integer address; off:
-    uint64[n+1] or None for uniform reads (n_reads x read_len).  -> (keys uint64[n, W] unsorted, n_windows_seen)."""
-    L = lib()
+def _sample_args(packed, off, pbits, parts, n_reads):
     if isinstance(packed, np.ndarray):
         packed = np.ascontiguousarray(packed, dtype=np.uint8)
         paddr = packed.ctypes.data
@@ -132,10 +131,19 @@ def sample_prefix(packed, off, K, pbits, parts, n_reads=None, read_len=0, n_thre
         oaddr = off.ctypes.data
     sel = np.zeros(1 << pbits, dtype=np.uint8)
     sel[np.asarray(list(parts), dtype=np.int64)] = 1
+    return (packed, off, sel), paddr, oaddr, n_reads
+
+
+def sample_prefix(packed, off, K, pbits, parts, n_reads=None, read_len=0, n_threads=0):
+    """Sampled-partition oracle, step 1 (SURVEY.md section 8c "human-scale check" ii): the canonical k-mer INSTANCES
+    of all reads whose leading `pbits` bits are one of `parts`.  packed: uint8 array or an integer address; off:
+    uint64[n+1] or None for uniform reads (n_reads x read_len).  -> (keys uint64[n, W] unsorted, n_windows_seen)."""
+    L = lib()
+    keep, paddr, oaddr, n_reads = _sample_args(packed, off, pbits, parts, n_reads)
     kp = C.POINTER(C.c_uint64)()
     n = C.c_uint64()
     nw = C.c_uint64()
-    rc = L.oracle_sample_prefix(paddr, oaddr, n_reads, read_len, K, pbits, sel.ctypes.data, n_threads,
+    rc = L.oracle_sample_prefix(paddr, oaddr, n_reads, read_len, K, pbits, keep[2].ctypes.data, n_threads,
                                 C.byref(kp), C.byref(n), C.byref(nw))
     if rc != 0:
         raise RuntimeError("oracle_sample_prefix failed rc=%d" % rc)
@@ -143,6 +151,29 @@ def sample_prefix(packed, off, K, pbits, parts, n_reads=None, read_len=0, n_thre
     keys = np.ctypeslib.as_array(kp, shape=(max(n.value, 1) * W,))[: n.value * W].copy().reshape(n.value, W)
     L.oracle_free(kp)
     return keys, nw.value
+
+
+def sample_prefix_pos(packed, off, K, pbits, parts, n_reads=None, read_len=0, n_threads=0):
+    """sample_prefix with where each instance sits: -> (keys uint64[n, W], pos uint64[n], n_windows_seen).
+    pos = (q << 1) | canonical_is_reverse, q = the window's first base in the packed stream (a palindrome counts as
+    forward): the encoding of apgk_occurrences_device.  Instances come ascending by q."""
+    L = lib()
+    keep, paddr, oaddr, n_reads = _sample_args(packed, off, pbits, parts, n_reads)
+    kp = C.POINTER(C.c_uint64)()
+    pp = C.POINTER(C.c_uint64)()
+    n = C.c_uint64()
+    nw = C.c_uint64()
+    rc = L.oracle_sample_prefix_pos(paddr, oaddr, n_reads, read_len, K, pbits, keep[2].ctypes.data, n_threads,
+                                    C.byref(kp), C.byref(pp), C.byref(n), C.byref(nw))
+    if rc != 0:
+        raise RuntimeError("oracle_sample_prefix_pos failed rc=%d" % rc)
+    W = n_words(K)
+    m = n.value
+    keys = np.ctypeslib.as_array(kp, shape=(max(m, 1) * W,))[: m * W].copy().reshape(m, W)
+    pos = np.ctypeslib.as_array(pp, shape=(max(m, 1),))[:m].copy()
+    L.oracle_free(kp)
+    L.oracle_free(pp)
+    return keys, pos, nw.value
 
 
 def count_keys(keys, K, n_threads=0):

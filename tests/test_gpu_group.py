@@ -99,6 +99,24 @@ def test_group_single_round(oracle, K, world, n_reads, empty, bucket_cost, monke
         kc.close()
 
 
+@pytest.mark.parametrize("K,prefix_bits,world,n_reads", [(26, 20, 1, 10_000), (26, 20, 3, 30_000)])
+def test_group_32bit_remainders_using_every_bit(oracle, K, prefix_bits, world, n_reads):
+    """prefix_bits = 2K - 32: the ranks exchange 4-byte remainders that use all 32 bits.  With several ranks the
+    gather splits them by their top split bits and the shards count the rest; one rank counts all 32 bits itself
+    (k_local2, not k_local3, which stops at REM = 31)."""
+    from allpathslg_b200 import KmerGroup
+
+    kcs, p, o = _make_ranks(oracle, K, world, n_reads, prefix_bits=prefix_bits)
+    with KmerGroup.local(kcs) as grp:
+        grp.count()
+        g, st = kcs[0].geometry(), grp.stats()
+        assert st["prefix_bits"] == prefix_bits and g["elem_bytes"] == 4
+        assert g["REM"] == 2 * K - prefix_bits - st["split_bits"]
+        _check_against_oracle(oracle, grp, kcs, p, o, K, sorted_by_rank=True)
+    for kc in kcs:
+        kc.close()
+
+
 @pytest.mark.parametrize("gather", ["direct", "pipelined"])
 @pytest.mark.parametrize("K,world,n_reads,outer_div,inner_div", [(25, 3, 30_000, 2, 5), (25, 2, 30_000, 1, 3), (48, 2, 12_000, 2, 4),
                                                                  (20, 4, 20_000, 3, 3), (96, 2, 6_000, 2, 2)])

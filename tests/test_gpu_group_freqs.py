@@ -104,7 +104,7 @@ def _check(got, exp):
                                                            (31, 2, 12_000, None, 0, 8), (48, 3, 12_000, None, 0, 16),
                                                            (96, 2, 8_000, 0, 0, 24), (25, 1, 10_000, None, 0, 8),
                                                            (25, 3, 30_000, None, 20, 4), (20, 2, 20_000, 1, 16, 4),
-                                                           (25, 1, 10_000, None, 20, 4)])
+                                                           (25, 1, 10_000, None, 20, 4), (26, 3, 30_000, None, 20, 4)])
 def test_group_read_freqs_match_the_oracle(oracle, K, world, n_reads, empty, pb, elem):
     """elem: the level-1 element the queries travel as -- a 4-byte remainder when the bits below the P-bit prefix
     fit (K = 20, or prefix_bits given: the table slices are searched in shared memory), else the one-word key (8

@@ -170,6 +170,78 @@ def test_huge_multiplicity_32bit_path(oracle):
         kc.close()
 
 
+_OCC_CHILD = (
+    "import sys, hashlib; sys.path.insert(0, %r)\n"
+    "import numpy as np\n"
+    "from allpathslg_b200 import KmerCounter\n"
+    "K, P = int(sys.argv[1]), int(sys.argv[2])\n"
+    "d = np.load(sys.argv[3])\n"
+    "kc = KmerCounter(K, prefix_bits=P); kc.add_reads(d['p'], d['o']); kc.finish(); kc.build_occurrences()\n"
+    "ro, rid, pos = kc.occurrences()\n"
+    "print(kc.geometry()['REM'], hashlib.sha256(ro.tobytes() + rid.tobytes() + pos.tobytes()).hexdigest())\n")
+
+
+@pytest.mark.parametrize("K,prefix_bits,rem", [(17, 2, 32), (22, 12, 32), (26, 20, 32), (28, 24, 32), (26, 21, 31)])
+def test_32bit_remainders_using_every_bit(oracle, K, prefix_bits, rem, tmp_path):
+    """4-byte level-1 elements whose remainder fills all 32 bits (P = 2K - 32): counted by k_local2 / k_local / k_big,
+    not k_local3, which takes REM <= 31 (its widest case, REM = 31, is the last row).  (17, 2) has 4 buckets, so
+    poly-A floods them past the shared-memory table and k_big runs on 32-bit remainders.  Table, spectrum, lookups,
+    read_freqs (bulk and per window) and occurrence records against the full oracle; the records both with remainder
+    and position packed in one word and, in a child process with APGK_OCC_NOPACK, in two arrays."""
+    import hashlib
+    import subprocess
+    import sys
+
+    rnd = random.Random(1000 + K)
+    reads = ["".join(rnd.choice("ACGT") for _ in range(rnd.choice([0, 1, K - 1, K, K + 1, K + 7, 150, 100])))
+             for _ in range(300)]
+    reads += ["A" * (K + 300), "ACGT" * 100, reads[3], "T" * (K + 20), "", "CG" * (K + 5)]
+    reads.append(reads[7].translate(RC)[::-1])
+    reads += ["A" * 200] * 20 + ["T" * 200] * 20 + ["ACGT" * 50] * 20
+    p, o = oracle.pack_strings(reads)
+    kc = _run(p, o, K, prefix_bits=prefix_bits)
+    g = kc.geometry()
+    assert (g["REM"], g["elem_bytes"]) == (rem, 4)
+    if (K, prefix_bits) == (17, 2):
+        assert g["n_big"] > 0
+    ek, ec = _assert_equal_to_oracle(oracle, kc, p, o, K)
+    en = int(ec.sum())
+    idx = np.random.RandomState(K).randint(0, len(ek), size=min(len(ek), 2000))
+    assert (kc.lookup(ek[idx], canonicalise=False).astype(np.uint64) == ec[idx]).all()
+    t, rc = ek[idx, 0].copy(), np.zeros(len(idx), dtype=np.uint64)   # the other strand of each k-mer
+    for _ in range(K):
+        rc = (rc << np.uint64(2)) | (np.uint64(3) - (t & np.uint64(3)))
+        t >>= np.uint64(2)
+    assert (kc.lookup(rc[:, None], canonicalise=True).astype(np.uint64) == ec[idx]).all()
+    q =np.random.RandomState(K + 1).randint(0, 2 ** 62, size=(2000, 1), dtype=np.int64).astype(np.uint64)
+    q[:, 0] &= np.uint64((1 << (2 * K)) - 1)
+    assert (kc.lookup(q, canonicalise=True).astype(np.uint64) == oracle.lookup(ek, ec, K, q, True)).all()
+    assert (kc.lookup(q, canonicalise=False).astype(np.uint64) == oracle.lookup(ek, ec, K, q, False)).all()
+    erf = oracle.read_freqs(p, o, K, ek, ec)
+    erf32 = np.where(erf == np.uint64(0xFFFFFFFFFFFFFFFF), np.uint64(0xFFFFFFFF), erf).astype(np.uint32)
+    tb = len(erf32)
+    assert (kc.read_freqs() == erf32).all()
+    assert (kc.read_freqs(0, tb - 1) == erf32[:tb - 1]).all()
+    assert (kc.read_freqs(17, tb - 30) == erf32[17:tb - 13]).all()
+    info = kc.build_occurrences()
+    assert info["n_occ"] == en
+    ero, erid, epos = oracle.occurrences(p, o, K, ek, en)
+    ro, rid, pos = kc.occurrences()
+    assert (ro == ero).all() and (rid == erid).all() and (pos == epos).all()
+    kc.close()
+    np.savez(tmp_path / "reads.npz", p=p, o=o)
+    env = dict(os.environ)
+    env.pop("APGK_OCC_DIRECT", None)
+    env["APGK_OCC_NOPACK"] = "1"
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "-c", _OCC_CHILD % root, str(K), str(prefix_bits), str(tmp_path / "reads.npz")],
+                       capture_output=True, text=True, env=env, timeout=600)
+    assert r.returncode == 0, r.stderr
+    got_rem, got_sha = r.stdout.split()
+    assert int(got_rem) == rem
+    assert got_sha == hashlib.sha256(ero.tobytes() + erid.tobytes() + epos.tobytes()).hexdigest()
+
+
 @pytest.mark.parametrize("K", [20, 25, 31, 48, 96])
 def test_kmer_space_rounds(oracle, K):
     """A small per-round budget forces several k-mer-space rounds (the SortKmers 'passes' / KmerParcels

@@ -171,3 +171,51 @@ def test_sampled_partition_oracle_matches_full_count(oracle, K):
     kr, nr = oracle.sample_prefix(pu, ou, K, pb, parts)
     assert nu == nr and (oracle.count_keys(ku, K)[0] == oracle.count_keys(kr, K)[0]).all()
     assert (oracle.count_keys(ku, K)[1] == oracle.count_keys(kr, K)[1]).all()
+
+
+def _prefix(kmers, K, pb):
+    """leading pb bits of each canonical k-mer (uint64[n, W] rows, most significant word first)"""
+    top = 2 * K - 64 * (kmers.shape[1] - 1)
+    if pb <= top:
+        return (kmers[:, 0] >> np.uint64(top - pb)).astype(np.int64)
+    return ((kmers[:, 0] << np.uint64(pb - top)) | (kmers[:, 1] >> np.uint64(64 - (pb - top)))).astype(np.int64)
+
+
+@pytest.mark.parametrize("K", [1, 16, 25, 33, 96])
+def test_sampled_partition_positions_match_full_records(oracle, K):
+    """oracle_sample_prefix_pos (what the wide-position GPU tests compare record by record where the full oracle cannot
+    run): its instances, sorted by (k-mer, position), are exactly the full oracle's occurrence records of the same
+    partitions, and every sampled window's count is the full oracle's read_freqs there -- ragged and uniform reads."""
+    rnd = random.Random(700 + K)
+    reads = ["".join(rnd.choice("ACGT") for _ in range(rnd.choice([0, 1, K - 1, K, K + 1, K + 9, 140]))) for _ in range(200)]
+    reads += ["A" * (K + 25), "ACGT" * 40, "T" * (K + 3), "", "CG" * (K + 4)]
+    reads.append(reads[5].translate(str.maketrans("ACGT", "TGCA"))[::-1])
+    sp = oracle.synth_params(100_000, 100)
+    pu, ou = oracle.synth_reads(sp, 0, 3_000)
+    pb = min(8, 2 * K)
+    parts = sorted({0, 5 % (1 << pb), 77 % (1 << pb), (1 << pb) - 1})
+    for p, o, uniform in ((*oracle.pack_strings(reads), False), (pu, ou, True)):
+        ek, ec, en = oracle.count(p, o, K)
+        ero, erid, epos = oracle.occurrences(p, o, K, ek, en)
+        if uniform:
+            keys, pos, nw = oracle.sample_prefix_pos(p, None, K, pb, parts, n_reads=len(o) - 1, read_len=100)
+        else:
+            keys, pos, nw = oracle.sample_prefix_pos(p, o, K, pb, parts)
+        assert nw == en
+        assert (keys == oracle.sample_prefix(p, o, K, pb, parts)[0]).all()    # the keys-only form sees the same instances
+        assert (np.diff(pos >> np.uint64(1)).astype(np.int64) > 0).all()      # ascending by position
+        # sort by (k-mer, position): a stable sort by k-mer keeps the position order
+        order = np.lexsort(keys.T[::-1]) if len(keys) else np.zeros(0, np.int64)
+        keys, pos = keys[order], pos[order]
+        m = np.isin(_prefix(ek, K, pb), parts)
+        inst = np.repeat(m, ec.astype(np.int64))
+        assert (keys == np.repeat(ek[m], ec[m].astype(np.int64), axis=0)).all()
+        q = (pos >> np.uint64(1)).astype(np.int64)
+        rid = np.searchsorted(o.astype(np.int64), q, side="right") - 1
+        p1 = q - o.astype(np.int64)[rid] + 1
+        assert (rid == erid[inst]).all()
+        assert (np.where(pos & np.uint64(1), -p1, p1) == epos[inst]).all()
+        sk, sc = oracle.count_keys(keys, K)
+        assert (sk == ek[m]).all() and (sc == ec[m]).all()
+        erf = oracle.read_freqs(p, o, K, ek, ec)
+        assert (erf[q] == np.repeat(sc, sc.astype(np.int64))).all()
