@@ -69,6 +69,10 @@ SYMBOLS = {
     "apgk_occurrences_info": (C.c_int, [_vp, _u64p, _u64p, C.POINTER(C.c_float)]),
     "apgk_occurrences_device": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), _u64p]),
     "apgk_occurrences_copy": (C.c_int, [_vp, C.c_uint64, C.c_uint64, _vp, _vp, _vp]),
+    "apgk_build_affixes": (C.c_int, [_vp, C.POINTER(C.c_float)]),
+    "apgk_affixes_device": (C.c_int, [_vp, C.POINTER(_vp), _u64p]),
+    "apgk_affixes_copy": (C.c_int, [_vp, C.c_uint64, C.c_uint64, _vp]),
+    "apgk_lookup_affixes": (C.c_int, [_vp, _vp, C.c_uint64, C.c_int, _vp, _vp]),
     "apgk_owner_plan": (C.c_int, [_vp, C.c_uint32, _vp]),
     "apgk_owner_scatter": (C.c_int, [_vp, _vp]),
     "apgk_key_buffer": (C.c_int, [_vp, C.c_uint64, C.POINTER(_vp)]),
@@ -116,6 +120,7 @@ SYMBOLS = {
     "apgk_debug_host_table_find": (C.c_int, [C.c_int, _vp, C.c_uint64, C.c_int, _vp, C.c_uint64, _vp]),
     "apgk_debug_host_splitters": (C.c_int, [_vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp]),
     "apgk_debug_host_synth": (C.c_int, [C.POINTER(SynthParams), C.c_uint64, C.c_uint64, _vp]),
+    "apgk_debug_host_affix_revcomp": (C.c_int, [_vp, C.c_uint64, _vp]),
 }
 
 _lib = None

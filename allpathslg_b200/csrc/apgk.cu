@@ -20,6 +20,7 @@
 
 #include "../../include/apgk.h"
 #include "gfreq.cuh"
+#include "affix.cuh"
 
 using namespace apgk;
 
@@ -107,6 +108,10 @@ struct apgk_ctx {
   uint64_t n_occ = 0, n_big_runs = 0;
   float occ_ms[5]{};
   float freq_ms[3]{};              // last bulk read_freqs: {memset + scan, sweep, placement}
+  // ---- affixes (apgk_build_affixes): one byte per distinct k-mer, a buffer of their own
+  DevBuf aff;
+  bool have_aff = false;
+  float aff_ms[3]{};               // last build: {clear + run-offset scan, sweep, per-bucket OR}
   cudaEvent_t occ_ev[6]{};
   std::vector<uint64_t> empty_nb;  // per read without bases: number of reads WITH bases before it
   uint64_t n_instances = 0, n_distinct = 0;
@@ -382,6 +387,7 @@ int append_bases(apgk_ctx* c, const uint8_t* packed, uint64_t first_base, uint64
 void invalidate_results(apgk_ctx* c) {
   c->finished = false; c->have_table = false; c->spec_loaded = false;
   c->table_from_reads = false; c->have_occ = false; c->n_occ = 0;
+  c->have_aff = false;
   c->n_instances = c->n_distinct = 0;
   c->owner_ranks = 0;
   c->part_ready = false; c->part_n = 0;
@@ -1384,6 +1390,89 @@ int read_freqs_bulk_dispatch(apgk_ctx* c, uint32_t* d_out) {
   return APGK_E_ARG;
 }
 
+// ---------------------------------------------------------------- affixes
+// The affix byte of every distinct k-mer into c->aff (n_distinct bytes, zeroed first): a sweep that sends every
+// window's element and affix byte to its prefix bucket's region, then one CTA per bucket ORs them into the rows.
+// The bucket regions are those of the occurrence records (occ_run_offsets + k_occ_bstart); A / B are reused.
+template <int W, typename Elem>
+int build_affixes_impl(apgk_ctx* c) {
+  const uint64_t N = c->n_instances, D = c->n_distinct;
+  const uint32_t nb = c->nb1;
+  constexpr bool U32 = sizeof(Elem) == 4;
+  c->have_aff = false;
+  for (float& m : c->aff_ms) m = 0;
+  { int rc = wait_ingest(c); if (rc) return rc; }
+  for (cudaEvent_t& e : c->occ_ev) if (!e) CU(cudaEventCreate(&e));
+  CU(c->aff.ensure(((D + 3) & ~3ull) + 4));
+  CU(cudaEventRecord(c->occ_ev[0], c->stream));
+  CU(cudaMemsetAsync(c->aff.p, 0, ((D + 3) & ~3ull) + 4, c->stream));
+  if (!N) {
+    CU(cudaStreamSynchronize(c->stream));
+    c->have_aff = true;
+    return APGK_OK;
+  }
+  { int rc = occ_run_offsets(c); if (rc) return rc; }
+  CU(c->occ_cnt.ensure(64));
+  unsigned long long* counters = c->occ_cnt.as<unsigned long long>();
+  CU(cudaMemsetAsync(counters, 0, 32, c->stream));
+  if (U32) {
+    CU(c->A.ensure(N * 8));
+  } else {
+    CU(c->A.ensure(N * sizeof(Key<W>)));
+    CU(c->B.ensure(N));
+  }
+  CU(c->occ_bstart.ensure(((size_t)nb + 1) * 8));
+  CU(c->occ_bcur.ensure((size_t)nb * 8));
+  k_occ_bstart<<<(nb + 1 + 255) / 256, 256, 0, c->stream>>>(c->out_off.as<unsigned long long>(), c->occ_off.as<unsigned long long>(),
+                                                         nb, c->occ_bstart.as<unsigned long long>(),
+                                                         c->occ_bcur.as<unsigned long long>());
+  LAUNCHED();
+  CU(cudaEventRecord(c->occ_ev[1], c->stream));
+  constexpr int NT = 128;
+  const uint64_t threads = (c->total_bases + POS_PER_THREAD - 1) / POS_PER_THREAD;
+  unsigned long long* elem64 = U32 ? c->A.as<unsigned long long>() : nullptr;
+  Key<W>* keys = U32 ? nullptr : c->A.as<Key<W>>();
+  uint8_t* bytes = U32 ? nullptr : c->B.as<uint8_t>();
+  k_aff_scatter<W, Elem, NT><<<(unsigned)((threads + NT - 1) / NT), NT, 0, c->stream>>>(
+      read_store(c), freq_table<W>(c), c->occ_bcur.as<unsigned long long>(), elem64, keys, bytes, N, counters);
+  LAUNCHED();
+  CU(cudaEventRecord(c->occ_ev[2], c->stream));
+  k_aff_place<W, Elem, OCC_PLACE_NT><<<std::min<uint32_t>(nb, (uint32_t)c->n_sm * 8), OCC_PLACE_NT, 0, c->stream>>>(
+      freq_table<W>(c), c->occ_bstart.as<unsigned long long>(), elem64, keys, bytes, c->aff.as<uint32_t>(), counters);
+  LAUNCHED();
+  CU(cudaEventRecord(c->occ_ev[3], c->stream));
+  unsigned long long h[3] = {0, 0, 0};
+  CU(cudaMemcpyAsync(h, counters, 24, cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  for (int i = 0; i < 3; i++) cudaEventElapsedTime(&c->aff_ms[i], c->occ_ev[i], c->occ_ev[i + 1]);
+  if (h[1] || h[2])
+    FAIL(APGK_E_STATE, "affixes: %llu windows missing from the table, %llu slots past a bucket (table does not match the read store)",
+         h[1], h[2]);
+  c->have_aff = true;
+  return APGK_OK;
+}
+
+template <int W>
+int lookup_affixes_impl(apgk_ctx* c, const uint64_t* kmers, uint64_t n, int canon, uint8_t* aff_out, uint32_t* counts_out) {
+  if (!n) return APGK_OK;
+  struct Tmp { DevBuf b; ~Tmp() { b.release(); } } q_, r_;   // released on every path out
+  DevBuf& q = q_.b; DevBuf& r = r_.b;
+  CU(q.ensure(n * sizeof(Key<W>)));
+  CU(r.ensure(n * 5));
+  uint32_t* d_cnt = r.as<uint32_t>();
+  uint8_t* d_aff = (uint8_t*)(d_cnt + n);
+  CU(cudaMemcpyAsync(q.p, kmers, n * sizeof(Key<W>), cudaMemcpyHostToDevice, c->stream));
+  k_lookup_affixes<W><<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(freq_table<W>(c), c->aff.as<uint8_t>(), q.as<Key<W>>(),
+                                                                         n, c->cfg.K, canon, d_aff, d_cnt);
+  c->launches++;
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpyAsync(aff_out, d_aff, n, cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess && counts_out) e = cudaMemcpyAsync(counts_out, d_cnt, n * 4, cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  CU(e);
+  return APGK_OK;
+}
+
 int occurrences_copy_impl(apgk_ctx* c, uint64_t first, uint64_t n_kmers, uint64_t* run_off_out, uint32_t* read_id_out,
                           int32_t* pos_out) {
   std::vector<unsigned long long> ends(2, 0);
@@ -1686,7 +1775,7 @@ void apgk_destroy(apgk_ctx* c) {
                    &c->big_list, &c->stats, &c->scratch, &c->stacks, &c->spec_dense, &c->spec_ovf, &c->misc, &c->deferred,
                    &c->out_keys, &c->out_cnt, &c->owner_plan_dev, &c->piece_off, &c->piece_tmp, &c->piece_ptrs, &c->C2, &c->sub_sizes, &c->TK,
                    &c->occ, &c->occ_pos, &c->occ_off, &c->occ_cnt, &c->occ_bstart, &c->occ_bcur, &c->rank_cnt, &c->rank_dir, &c->empty_dev,
-                   &c->occ_tmp};
+                   &c->occ_tmp, &c->aff};
   for (DevBuf* b : all) b->release();
   for (cudaEvent_t e : c->occ_ev) if (e) cudaEventDestroy(e);
   for (auto& iv : c->ivs) { cudaEventDestroy(iv.e0); cudaEventDestroy(iv.e1); }
@@ -2094,7 +2183,7 @@ int apgk_reserve_table(apgk_ctx* c, uint64_t n_records) {
     c->out_keys.release(); c->out_cnt.release();
     CU(c->out_keys.ensure(std::max<size_t>(n_records, 1) * kb));
     CU(c->out_cnt.ensure(std::max<size_t>(n_records, 1) * 4));
-    c->have_table = false;
+    c->have_table = false; c->have_aff = false;
   }
   return APGK_OK;
 }
@@ -2224,6 +2313,65 @@ int apgk_read_freqs_device(apgk_ctx* c, uint32_t* d_out, float* ms3) {
   }
   if (ms3) for (int i = 0; i < 3; i++) ms3[i] = c->freq_ms[i];
   return rc;
+}
+
+int apgk_build_affixes(apgk_ctx* c, float* ms3) {
+  if (!c) return APGK_E_ARG;
+  if (!c->finished || !c->have_table || !(c->cfg.flags & APGK_WANT_COUNTS))
+    FAIL(APGK_E_STATE, "no table: finish with APGK_WANT_COUNTS first");
+  if (!c->table_from_reads)
+    FAIL(APGK_E_STATE, "affixes need a table counted from this context's read store (apgk_finish, not a shard or a key array)");
+  CU(cudaSetDevice(c->device));
+  int rc = APGK_E_ARG;
+  switch (c->W) {
+    case 1: rc = c->geom.REM <= 32 ? build_affixes_impl<1, uint32_t>(c) : build_affixes_impl<1, Key<1>>(c); break;
+    case 2: rc = build_affixes_impl<2, Key<2>>(c); break;
+    case 3: rc = build_affixes_impl<3, Key<3>>(c); break;
+  }
+  if (ms3) for (int i = 0; i < 3; i++) ms3[i] = c->aff_ms[i];
+  return rc;
+}
+
+// the affixes of the current table, or why there are none
+static int affixes_ready(apgk_ctx* c) {
+  if (!c->finished || !c->have_table || !(c->cfg.flags & APGK_WANT_COUNTS))
+    FAIL(APGK_E_STATE, "no table: finish with APGK_WANT_COUNTS first");
+  if (!c->table_from_reads)
+    FAIL(APGK_E_STATE, "affixes need a table counted from this context's read store (apgk_finish, not a shard or a key array)");
+  if (!c->have_aff) FAIL(APGK_E_STATE, "no affixes: call apgk_build_affixes first");
+  return APGK_OK;
+}
+
+int apgk_affixes_device(apgk_ctx* c, const uint8_t** d_aff, uint64_t* n_distinct) {
+  if (!c) return APGK_E_ARG;
+  { int rc = affixes_ready(c); if (rc) return rc; }
+  if (d_aff) *d_aff = c->aff.as<uint8_t>();
+  if (n_distinct) *n_distinct = c->n_distinct;
+  return APGK_OK;
+}
+
+int apgk_affixes_copy(apgk_ctx* c, uint64_t first, uint64_t n, uint8_t* out) {
+  if (!c || (!out && n)) return APGK_E_ARG;
+  { int rc = affixes_ready(c); if (rc) return rc; }
+  if (first > c->n_distinct || n > c->n_distinct - first) FAIL(APGK_E_ARG, "range beyond the table");
+  if (!n) return APGK_OK;
+  CU(cudaSetDevice(c->device));
+  CU(cudaMemcpyAsync(out, c->aff.as<uint8_t>() + first, n, cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return APGK_OK;
+}
+
+int apgk_lookup_affixes(apgk_ctx* c, const uint64_t* kmers, uint64_t n, int canonicalise, uint8_t* aff_out,
+                        uint32_t* counts_out) {
+  if (!c || (!kmers && n) || (!aff_out && n)) return APGK_E_ARG;
+  { int rc = affixes_ready(c); if (rc) return rc; }
+  CU(cudaSetDevice(c->device));
+  switch (c->W) {
+    case 1: return lookup_affixes_impl<1>(c, kmers, n, canonicalise, aff_out, counts_out);
+    case 2: return lookup_affixes_impl<2>(c, kmers, n, canonicalise, aff_out, counts_out);
+    case 3: return lookup_affixes_impl<3>(c, kmers, n, canonicalise, aff_out, counts_out);
+  }
+  return APGK_E_ARG;
 }
 
 int apgk_owner_plan(apgk_ctx* c, uint32_t n_ranks, uint64_t* counts_out) {
@@ -2492,6 +2640,12 @@ int apgk_debug_host_canonical(int K, const uint64_t* kmers, uint64_t n, uint64_t
     else if (W == 2) { Key<2> k; memcpy(k.w, kmers + 2 * i, 16); k = key_canonical(k, K); memcpy(out + 2 * i, k.w, 16); }
     else { Key<3> k; memcpy(k.w, kmers + 3 * i, 24); k = key_canonical(k, K); memcpy(out + 3 * i, k.w, 24); }
   }
+  return APGK_OK;
+}
+
+int apgk_debug_host_affix_revcomp(const uint8_t* aff, uint64_t n, uint8_t* out) {
+  if ((!aff || !out) && n) return APGK_E_ARG;
+  for (uint64_t i = 0; i < n; i++) out[i] = (uint8_t)aff_revcomp(aff[i]);
   return APGK_OK;
 }
 

@@ -231,6 +231,40 @@ class KmerCounter:
         self._ck(self._L.apgk_occurrences_device(self._h, C.byref(a), C.byref(b), C.byref(n)))
         return a.value, b.value, n.value
 
+    # -- affixes: which bases precede (bits 0-3) and follow (bits 4-7) every distinct k-mer, canonical orientation
+    def build_affixes(self):
+        """Sweep of the read store that ORs every window's neighbour bases into its k-mer's affix byte (needs
+        finish() with want_counts).  -> device ms {scan, sweep, place}."""
+        ms = (C.c_float * 3)()
+        self._ck(self._L.apgk_build_affixes(self._h, ms))
+        return dict(zip(("scan", "sweep", "place"), [float(x) for x in ms]))
+
+    def affixes(self, first=0, n=None):
+        """-> uint8[n]: the affix bytes of rows [first, first+n) of the sorted table."""
+        _, nd = self.totals()
+        if n is None:
+            n = nd - first
+        out = np.zeros(max(n, 1), dtype=np.uint8)
+        self._ck(self._L.apgk_affixes_copy(self._h, first, n, out.ctypes.data))
+        return out[:n]
+
+    def affixes_device(self):
+        """-> (device pointer of uint8[n_distinct], n_distinct)"""
+        p = C.c_void_p()
+        n = C.c_uint64()
+        self._ck(self._L.apgk_affixes_device(self._h, C.byref(p), C.byref(n)))
+        return p.value, n.value
+
+    def lookup_affixes(self, kmers, canonicalise=True):
+        """-> (affixes uint8[n] in each query's own orientation, counts uint32[n]); absent k-mers give (0, 0)."""
+        q = np.ascontiguousarray(kmers, dtype=np.uint64)
+        n = q.size // self.W
+        aff = np.zeros(max(n, 1), dtype=np.uint8)
+        cnt = np.zeros(max(n, 1), dtype=np.uint32)
+        self._ck(self._L.apgk_lookup_affixes(self._h, q.ctypes.data, n, 1 if canonicalise else 0, aff.ctypes.data,
+                                             cnt.ctypes.data))
+        return aff[:n], cnt[:n]
+
     # -- multi-GPU building blocks
     def owner_plan(self, n_ranks):
         out = np.zeros(n_ranks, dtype=np.uint64)

@@ -21,6 +21,8 @@
  *                           KmerParcelReader batches, KmerKmerFreq vectors [U]
  *   apgk_*occurrences*   <- the (read id, signed position) payload of SortKmers' kmer records and
  *                           KmerParcels' batches (src/kmers/KmerRecord.h, kmer_parcels/ [U])
+ *   apgk_*affixes*       <- the affixes of naif_kmer's "k-mer + frequency + affixes" records
+ *                           (KmerFreqAffixes, src/kmers/naif_kmer/ [U])
  *   apgk_lookup*, apgk_read_freqs*
  *                        <- the k-mer frequency tables FindErrors queries per read
  *                           position (src/paths/FindErrors*.cc [BJ name, U path])
@@ -176,6 +178,40 @@ int apgk_occurrences_device(apgk_ctx* ctx, const uint64_t** d_run_off, const uin
  * NULL = offsets only, to size the buffers). */
 int apgk_occurrences_copy(apgk_ctx* ctx, uint64_t first_kmer, uint64_t n_kmers, uint64_t* run_off_out,
                           uint32_t* read_id_out, int32_t* pos_out);
+
+/* ---- k-mer affixes: which bases precede and which follow every distinct k-mer in the reads -- the "k-mer +
+ * frequency + affixes" record of the reference's naif_kmer layer (KmerFreqAffixes [U]), what the unipath / graph
+ * code reads per k-mer: with it the de Bruijn graph follows from the table without a second pass over the reads.
+ * Definition.  For the window instance x at base p of a read (forward, as read): L = the base at p-1 unless p is
+ * the read's first base, R = the base at p+K if that base is in the same read (otherwise none).  With
+ * c = canonical(x), the instance sets
+ *   x <  revcomp(x) (c is forward):                pre(c) |= L,        suf(c) |= R
+ *   x >  revcomp(x) (c is the reverse complement): pre(c) |= comp(R),  suf(c) |= comp(L)
+ *   x == revcomp(x) (palindrome, even K only):     both of the above, so a palindrome's affix set is closed under
+ *                                                  reverse complement (unlike the occurrence records, where a
+ *                                                  palindrome counts as forward: a graph builder needs both).
+ * Equivalently: bit (c, suf, b) is set iff the (K+1)-mer c.b or its reverse complement occurs in the reads, bit
+ * (c, pre, b) iff b.c or its reverse complement does.
+ * Encoding: one byte per distinct k-mer, row i of the sorted table (apgk_counts_copy row i); bit b (0..3) = base b
+ * (A, C, G, T) precedes c, bit 4+b = base b follows c.
+ * apgk_build_affixes needs a context finished by apgk_finish with APGK_WANT_COUNTS, its read store in place (the same
+ * precondition as apgk_build_occurrences): APGK_E_STATE otherwise, also on a shard after apgk_group_count and after
+ * apgk_finish_keys_device / apgk_count_pieces*; APGK_E_RANGE when a count saturated.  ms3 (may be NULL) = device
+ * milliseconds of {clear + run-offset scan, sweep of the reads, per-bucket OR}.  The affixes live in a buffer of their
+ * own: they survive apgk_release_temp, apgk_build_occurrences and apgk_read_freqs*, and are dropped by whatever
+ * drops the table (apgk_add_reads*, apgk_finish*, apgk_reset, apgk_group_count).  The other three calls refuse with
+ * APGK_E_STATE before apgk_build_affixes. */
+int apgk_build_affixes(apgk_ctx* ctx, float* ms3);
+/* DEVICE pointer (n_distinct bytes), library-owned until the table is dropped. */
+int apgk_affixes_device(apgk_ctx* ctx, const uint8_t** d_aff, uint64_t* n_distinct);
+/* HOST copy of rows [first, first+n); APGK_E_ARG for a range beyond the table. */
+int apgk_affixes_copy(apgk_ctx* ctx, uint64_t first, uint64_t n, uint8_t* out);
+/* Affixes of arbitrary k-mers (host arrays, W words each), in the QUERY's orientation: when canonicalise != 0 and
+ * query q is the reverse complement of its canonical form c, pre(q) = comp(suf(c)) and suf(q) = comp(pre(c)) (swap
+ * the nibbles, base bit b -> 3-b).  Absent k-mers give 0; counts_out (may be NULL) tells absent (0) from
+ * present-without-neighbours. */
+int apgk_lookup_affixes(apgk_ctx* ctx, const uint64_t* kmers, uint64_t n, int canonicalise, uint8_t* aff_out,
+                        uint32_t* counts_out);
 
 /* ---- multi-GPU building blocks (one context per rank; the exchange itself is the caller's,
  * e.g. NCCL all-to-all).  Canonical k-mers are owned by rank hash(kmer) % n_ranks. */
@@ -356,6 +392,9 @@ int apgk_debug_host_topdigits(const uint8_t* packed, const uint64_t* off, uint64
 int apgk_debug_host_table_find(int K, const uint64_t* sorted_kmers, uint64_t n, int prefix_bits, const uint64_t* queries,
                                uint64_t n_q, uint64_t* idx_out);
 int apgk_debug_host_synth(const apgk_synth_params* p, uint64_t r0, uint64_t n_reads, uint8_t* packed_out);
+/* The orientation transform of apgk_lookup_affixes on the HOST: out[i] = affix byte of the reverse complement of a
+ * k-mer whose affix byte is aff[i]. */
+int apgk_debug_host_affix_revcomp(const uint8_t* aff, uint64_t n, uint8_t* out);
 /* The sharded form's ownership rule on the HOST: bounds_out[world + 1] = the contiguous bucket ranges of equal cost
  * (cost of a non-empty bucket = its size + bucket_cost; bucket_cost 0 = equal instance counts) that the device's
  * k_total_sizes -> scan -> k_splitters derive from the all-gathered bucket sizes. */

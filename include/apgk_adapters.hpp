@@ -195,12 +195,49 @@ class KmerParcelsBuilder {
     e_.ck(apgk_occurrences_copy(e_.ctx(), first, n, nullptr, read_ids.data(), positions.data()));
     read_ids.resize(m); positions.resize(m);
   }
+  // affixes of k-mers [first, first+n): out[i] = bases preceding (bits 0-3) and following (bits 4-7) k-mer first+i
+  void Affixes(uint64_t first, uint64_t n, uint8_t* out) {
+    if (!aff_) { e_.ck(apgk_build_affixes(e_.ctx(), nullptr)); aff_ = true; }
+    e_.ck(apgk_affixes_copy(e_.ctx(), first, n, out));
+  }
   const Engine& engine() const { return e_; }
 
  private:
   Engine e_;
-  bool built_ = false, occ_ = false;
+  bool built_ = false, occ_ = false, aff_ = false;
 };
+
+// One record of naif_kmer's "k-mer + frequency + affixes" kind (KmerFreqAffixes [U]): bit b of affixes = base b
+// precedes the canonical k-mer somewhere in the reads, bit 4+b = base b follows it (include/apgk.h).
+template <int W>
+struct kmer_freq_affixes {
+  uint64_t kmer[W];
+  uint32_t count;
+  uint8_t affixes;
+};
+
+// `KmerFreqAffixes`: every distinct canonical k-mer, ascending, with its count and affixes.
+template <int K>
+void KmerFreqAffixes(const vecbasevector& reads, std::vector<kmer_freq_affixes<(2 * K + 63) / 64>>& R, int device = 0) {
+  constexpr int W = (2 * K + 63) / 64;
+  Engine e(K, /*want_counts=*/true, device);
+  e.AddReads(reads);
+  e.Finish();
+  e.ck(apgk_build_affixes(e.ctx(), nullptr));
+  uint64_t ni = 0, nd = 0;
+  e.ck(apgk_totals(e.ctx(), &ni, &nd));
+  std::vector<uint64_t> k(nd * W + 1);
+  std::vector<uint32_t> c(nd + 1);
+  std::vector<uint8_t> a(nd + 1);
+  e.ck(apgk_counts_copy(e.ctx(), 0, nd, k.data(), c.data()));
+  e.ck(apgk_affixes_copy(e.ctx(), 0, nd, a.data()));
+  R.resize(nd);
+  for (uint64_t i = 0; i < nd; i++) {
+    for (int j = 0; j < W; j++) R[i].kmer[j] = k[i * W + j];
+    R[i].count = c[i];
+    R[i].affixes = a[i];
+  }
+}
 
 // The k-mer frequency table error correction queries.
 class KmerFreqTable {
