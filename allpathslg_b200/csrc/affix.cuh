@@ -34,15 +34,21 @@ __device__ __forceinline__ void aff_or_byte(uint32_t* __restrict__ aff32, unsign
 
 // Sweep of the reads: every valid window takes the next slot of its prefix bucket and stores its element with
 // its affix byte there.  U32 elements: elem64[o] = rem << 8 | affix.  Full keys: keys[o] = key, bytes[o] = affix.
+// Only the windows starting in [first, first + n_bases) take part (the whole store on one GPU, a batch of it in the
+// group build, gaffix.cuh); their neighbours are read from the store itself, so a batch's edges change no byte.
 template <int W, typename Elem, int NT>
-__global__ void __launch_bounds__(NT) k_aff_scatter(ReadStore rs, FreqTable<W> t, unsigned long long* __restrict__ bcur,
+__global__ void __launch_bounds__(NT) k_aff_scatter(ReadStore rs, FreqTable<W> t, uint64_t first, uint64_t n_bases,
+                                                    unsigned long long* __restrict__ bcur,
                                                     unsigned long long* __restrict__ elem64, Key<W>* __restrict__ keys,
                                                     uint8_t* __restrict__ bytes, unsigned long long n_slots,
                                                     unsigned long long* __restrict__ counters) {
   constexpr bool U32 = sizeof(Elem) == 4;
-  const uint64_t p = ((uint64_t)blockIdx.x * NT + threadIdx.x) * POS_PER_THREAD;
-  if (p >= rs.total_bases) return;
-  const uint32_t valid = window_valid_mask16(rs.starts32, p, rs.K, rs.total_bases);
+  const uint64_t p = (first & ~15ull) + ((uint64_t)blockIdx.x * NT + threadIdx.x) * POS_PER_THREAD;
+  const uint64_t end = first + n_bases;
+  if (p >= end) return;
+  uint32_t valid = window_valid_mask16(rs.starts32, p, rs.K, rs.total_bases);
+  if (p < first) valid &= 0xFFFFu << (uint32_t)(first - p);
+  if (end - p < 16) valid &= (1u << (uint32_t)(end - p)) - 1u;
   if (!valid) return;
   Window16<W> win;
   load_window16<W>(rs.bases32, p, rs.K, win);

@@ -21,6 +21,7 @@
 #include "../../include/apgk.h"
 #include "gfreq.cuh"
 #include "affix.cuh"
+#include "gaffix.cuh"
 
 using namespace apgk;
 
@@ -111,6 +112,7 @@ struct apgk_ctx {
   // ---- affixes (apgk_build_affixes): one byte per distinct k-mer, a buffer of their own
   DevBuf aff;
   bool have_aff = false;
+  bool aff_group = false;          // the affixes of a shard, built by apgk_group_build_affixes over all ranks' reads
   float aff_ms[3]{};               // last build: {clear + run-offset scan, sweep, per-bucket OR}
   cudaEvent_t occ_ev[6]{};
   std::vector<uint64_t> empty_nb;  // per read without bases: number of reads WITH bases before it
@@ -387,7 +389,7 @@ int append_bases(apgk_ctx* c, const uint8_t* packed, uint64_t first_base, uint64
 void invalidate_results(apgk_ctx* c) {
   c->finished = false; c->have_table = false; c->spec_loaded = false;
   c->table_from_reads = false; c->have_occ = false; c->n_occ = 0;
-  c->have_aff = false;
+  c->have_aff = false; c->aff_group = false;
   c->n_instances = c->n_distinct = 0;
   c->owner_ranks = 0;
   c->part_ready = false; c->part_n = 0;
@@ -1434,7 +1436,7 @@ int build_affixes_impl(apgk_ctx* c) {
   Key<W>* keys = U32 ? nullptr : c->A.as<Key<W>>();
   uint8_t* bytes = U32 ? nullptr : c->B.as<uint8_t>();
   k_aff_scatter<W, Elem, NT><<<(unsigned)((threads + NT - 1) / NT), NT, 0, c->stream>>>(
-      read_store(c), freq_table<W>(c), c->occ_bcur.as<unsigned long long>(), elem64, keys, bytes, N, counters);
+      read_store(c), freq_table<W>(c), 0, c->total_bases, c->occ_bcur.as<unsigned long long>(), elem64, keys, bytes, N, counters);
   LAUNCHED();
   CU(cudaEventRecord(c->occ_ev[2], c->stream));
   k_aff_place<W, Elem, OCC_PLACE_NT><<<std::min<uint32_t>(nb, (uint32_t)c->n_sm * 8), OCC_PLACE_NT, 0, c->stream>>>(
@@ -2336,9 +2338,10 @@ int apgk_build_affixes(apgk_ctx* c, float* ms3) {
 static int affixes_ready(apgk_ctx* c) {
   if (!c->finished || !c->have_table || !(c->cfg.flags & APGK_WANT_COUNTS))
     FAIL(APGK_E_STATE, "no table: finish with APGK_WANT_COUNTS first");
-  if (!c->table_from_reads)
-    FAIL(APGK_E_STATE, "affixes need a table counted from this context's read store (apgk_finish, not a shard or a key array)");
-  if (!c->have_aff) FAIL(APGK_E_STATE, "no affixes: call apgk_build_affixes first");
+  if (!c->table_from_reads && !c->aff_group)
+    FAIL(APGK_E_STATE, "affixes need a table counted from this context's read store (apgk_finish, not a key array), or a shard "
+                       "after apgk_group_build_affixes");
+  if (!c->have_aff) FAIL(APGK_E_STATE, "no affixes: call apgk_build_affixes (apgk_group_build_affixes on a shard) first");
   return APGK_OK;
 }
 
@@ -2568,6 +2571,11 @@ int apgk_group_read_freqs_device(apgk_group* g, uint32_t* const* d_out, const ui
                                  apgk_group_freq_stats* stats) {
   if (!g) return APGK_E_ARG;
   return group_read_freqs(g, d_out, first_base, n_bases, stats);
+}
+
+int apgk_group_build_affixes(apgk_group* g, apgk_group_affix_stats* stats) {
+  if (!g) return APGK_E_ARG;
+  return group_build_affixes(g, stats);
 }
 
 int apgk_group_totals(const apgk_group* g, uint64_t* n_instances, uint64_t* n_distinct) {

@@ -853,10 +853,57 @@ int group_count(apgk_group* g) {
 // ---------------------------------------------------------------- frequency lookups on the sharded table
 // apgk_group_read_freqs_device; the kernels and the data flow are described in gfreq.cuh.
 
-struct FreqMeta {   // what every rank tells the others before a lookup (all-gathered, host side)
+struct FreqMeta {   // what every rank tells the others before a lookup or an affix build (all-gathered, host side)
   int32_t status, pad_;   // 0, or the error this rank met while preparing
   uint64_t n_bases, batch_bases, cap_B, cap_sub, ptr_B, ptr_sub;
 };
+
+// Bytes of B one batch of n bases takes: the level-1 elements (eb bytes), and for the affix build (gaffix.cuh) their
+// affix bytes -- one u64 per slot with a 4-byte remainder, else a byte plane behind the keys at a 16-byte aligned
+// offset (aff_plane), inside the same exported buffer.
+uint64_t aff_plane(uint64_t n, uint64_t eb) { return eb == 4 ? 0 : (n * eb + 15) & ~15ull; }
+uint64_t exchange_B_bytes(uint64_t n, uint64_t eb, bool aff) { return (!aff ? n * eb : eb == 4 ? n * 8 : aff_plane(n, eb) + n) + 16; }
+
+// The preparation the exchanges over a rank's read store share (the lookups and the affix build), in two steps around
+// the caller's own allocations (the lookups' positions, the affix array), so that the check whether B can grow sees
+// the memory those took.  exchange_batch: the batch size from the budget of the count's temp buffers -- per base at
+// most one element in B and 4 more bytes (the lookups' position; the affix byte, or the u64 slot of a 4-byte
+// remainder, fits in them).  exchange_buffers: the buffers of a batch, then whether B can grow to hold one.  It must
+// come after every other allocation of the preparation: B grows later, after a collective, where a rank that failed
+// alone would leave the others waiting.
+void exchange_batch(apgk_group* g, int i, FreqMeta& m) {
+  apgk_ctx* c = g->rs[i].c;
+  uint64_t budget = c->budget_bytes;
+  if (const char* e = getenv("APGK_BUDGET_BYTES")) { if (atoll(e) > 0) budget = (uint64_t)atoll(e); }   // tests: a small device
+  m.batch_bases = std::min<uint64_t>(std::max<uint64_t>(budget / (c->elem_bytes + 4), 4096), 1ull << 31) & ~15ull;
+}
+
+int exchange_buffers(apgk_group* g, int i, bool aff, FreqMeta& m) {
+  RankState& r = g->rs[i];
+  apgk_ctx* c = r.c;
+  const int me = g->rank0 + i;
+  const uint64_t per = std::min(m.batch_bases, m.n_bases);
+  const uint32_t nb = r.nb;
+  const int world = g->world;
+  GCU(r.gcnt.ensure(64));
+  GCU(c->piece_off.ensure((size_t)world * ((size_t)nb + 1) * 8));
+  GCU(r.sizes32.ensure((size_t)nb * 4));
+  GCU(r.sizes_all.ensure((size_t)world * nb * 4));
+  GCU(c->occ_bcur.ensure((size_t)nb * 8));
+  GCU(r.ptrs_dev.ensure(3 * (size_t)world * 8));
+  GCU(r.red_out.ensure(64));
+  GCU(c->blocksum.ensure((((size_t)nb + 1 + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * 8));   // what scan_u32 takes
+  for (cudaEvent_t& e : r.gev) if (!e) GCU(cudaEventCreate(&e));
+  // B grows later, in refresh_exports (peers may have it mapped): here only whether it can
+  const uint64_t need_B = exchange_B_bytes(per, c->elem_bytes, aff);
+  if (need_B > c->B.cap) {
+    size_t fr = 0, tot = 0;
+    GCU(cudaMemGetInfo(&fr, &tot));
+    if ((uint64_t)fr + c->B.cap < need_B + (64ull << 20))
+      GFAIL(APGK_E_NOMEM, "rank %d: the partition buffer needs %llu bytes, %llu free", me, (unsigned long long)need_B, (unsigned long long)fr);
+  }
+  return APGK_OK;
+}
 
 // Everything that can fail on one rank alone is decided here, before the call's first collective, and travels to
 // the others in FreqMeta::status: a rank that failed on its own between two collectives would leave the others
@@ -879,43 +926,28 @@ int gfreq_prepare(apgk_group* g, int i, uint32_t* const* d_out, const uint64_t* 
   if (n_bases[i] && !d_out[i]) GFAIL(APGK_E_ARG, "rank %d: no output buffer", me);
   m.n_bases = n_bases[i];
   GCU(cudaSetDevice(c->device));
-  // batch size from the budget of the count's temp buffers: per base at most one element in B and one position
-  uint64_t budget = c->budget_bytes;
-  if (const char* e = getenv("APGK_BUDGET_BYTES")) { if (atoll(e) > 0) budget = (uint64_t)atoll(e); }   // tests: a small device
-  const uint64_t eb = c->elem_bytes;
-  m.batch_bases = std::min<uint64_t>(std::max<uint64_t>(budget / (eb + 4), 4096), 1ull << 31) & ~15ull;
-  const uint64_t per = std::min(m.batch_bases, m.n_bases);
-  const uint32_t nb = r.nb;
-  const int world = g->world;
-  GCU(r.gpos.ensure(std::max<uint64_t>(per, 1) * 4));
-  GCU(r.gcnt.ensure(64));
-  GCU(c->piece_off.ensure((size_t)world * ((size_t)nb + 1) * 8));
-  GCU(r.sizes32.ensure((size_t)nb * 4));
-  GCU(r.sizes_all.ensure((size_t)world * nb * 4));
-  GCU(c->occ_bcur.ensure((size_t)nb * 8));
-  GCU(r.ptrs_dev.ensure(3 * (size_t)world * 8));
-  GCU(r.red_out.ensure(64));
-  GCU(c->blocksum.ensure((((size_t)nb + 1 + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * 8));   // what scan_u32 takes
-  for (cudaEvent_t& e : r.gev) if (!e) GCU(cudaEventCreate(&e));
-  // B grows later, in refresh_exports (peers may have it mapped): here only whether it can
-  const uint64_t need_B = per * eb + 16;
-  if (need_B > c->B.cap) {
-    size_t fr = 0, tot = 0;
-    GCU(cudaMemGetInfo(&fr, &tot));
-    if ((uint64_t)fr + c->B.cap < need_B + (64ull << 20))
-      GFAIL(APGK_E_NOMEM, "rank %d: the partition buffer needs %llu bytes, %llu free", me, (unsigned long long)need_B, (unsigned long long)fr);
-  }
-  return APGK_OK;
+  exchange_batch(g, i, m);
+  GCU(r.gpos.ensure(std::max<uint64_t>(std::min(m.batch_bases, m.n_bases), 1) * 4));
+  return exchange_buffers(g, i, false, m);
 }
 
-template <int W, typename Elem>
-int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base, const std::vector<FreqMeta>& meta,
-                           apgk_group_freq_stats* st) {
+// The batch loop both exchanges over the ranks' read stores run (the lookups and the affix build; the kernels are
+// described in gfreq.cuh and gaffix.cuh).  Every rank's B is grown and re-exported to hold one batch (need_B(s) bytes
+// for rank s), then, per batch of BB bases of every local rank's range [first_base[i], + meta.n_bases):
+//   sender  the batch's windows counted by coarse bucket into sizes32 (k_occ_scatter), scanned into the rank's own
+//           piece offsets and the bucket cursors; place(i, b0, first, nbb, tp, grid) puts the elements into B
+//   all     the bucket sizes all-gathered, every other source's piece offsets scanned
+//   owner   own(i, ts) runs the owner kernel over the rank's owned segments
+//   all     a barrier: the owners are done with every B (the next batch may overwrite it)
+//   sender  after(i, b0, nbb)
+// start(i) runs once per local rank after the call's start event; counters[4] (r.gcnt) are summed over the ranks at
+// the end into red, the first local rank's own into own; ms[3] = device times {sweep, exchange, after} of the first
+// local context, summed over the batches, *total_ms the whole call.
+template <int W, typename Elem, typename NeedB, typename Start, typename Place, typename Own, typename After>
+int exchange_batches(apgk_group* g, const std::vector<FreqMeta>& meta, const uint64_t* first_base, uint64_t BB, uint64_t n_batches,
+                     NeedB need_B_of, Start start, Place place, Own own, After after, unsigned long long red[4],
+                     unsigned long long own_cnt[4], float ms[3], float* total_ms) {
   const int world = g->world, nl = g->n_local;
-  constexpr uint64_t eb = sizeof(Elem);
-  uint64_t BB = ~0ull, n_batches = 0;
-  for (int s = 0; s < world; s++) BB = std::min<uint64_t>(BB, meta[s].batch_bases);
-  for (int s = 0; s < world; s++) n_batches = std::max<uint64_t>(n_batches, (meta[s].n_bases + BB - 1) / BB);
   // every rank's B large enough for one batch, re-exported where it grew (after apgk_release_temp too)
   {
     std::vector<GroupMeta> gm(world);
@@ -923,7 +955,7 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
     for (int s = 0; s < world; s++) {
       gm[s] = GroupMeta{};
       gm[s].cap_B = meta[s].cap_B; gm[s].cap_sub = meta[s].cap_sub; gm[s].ptr_B = meta[s].ptr_B; gm[s].ptr_sub = meta[s].ptr_sub;
-      need_B[s] = std::min(BB, meta[s].n_bases) * eb + 16;
+      need_B[s] = need_B_of(s);
     }
     int rc = refresh_exports(g, gm, need_B, 16);
     if (rc) return rc;
@@ -939,7 +971,12 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
   }
   GCU(cudaSetDevice(c0->device));
   GCU(cudaEventRecord(r0.gev[4], c0->stream));
-  float ms[3] = {0, 0, 0};
+  for (int i = 0; i < nl; i++) {
+    GCU(cudaSetDevice(g->rs[i].c->device));
+    int rc = start(i);
+    if (rc) return rc;
+  }
+  ms[0] = ms[1] = ms[2] = 0;
   auto collect = [&]() {   // stage times of the batch just run, first local context
     cudaEventSynchronize(r0.gev[3]);
     for (int k = 0; k < 3; k++) { float x = 0; if (cudaEventElapsedTime(&x, r0.gev[k], r0.gev[k + 1]) == cudaSuccess) ms[k] += x; }
@@ -947,7 +984,7 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
   constexpr int NT = 128;
   for (uint64_t k = 0; k < n_batches; k++) {
     if (k) collect();
-    // -- sender: histogram of the batch's windows by coarse bucket, bucket starts, elements into B
+    // -- sender: histogram of the batch's windows by coarse bucket, bucket starts, then the caller's placement
     for (int i = 0; i < nl; i++) {
       RankState& r = g->rs[i];
       apgk_ctx* c = r.c;
@@ -956,33 +993,29 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
       if (i == 0) GCU(cudaEventRecord(r.gev[0], c->stream));
       const uint32_t nb = r.nb;
       const uint64_t n = meta[me].n_bases, b0 = std::min(k * BB, n), nbb = std::min(BB, n - b0), first = first_base[i] + b0;
-      FreqTable<W> tp{};   // the partition geometry: the sweep reads only the bucket digit's position
+      FreqTable<W> tp{};   // the partition geometry: the sweeps read only the bucket digit's position
       tp.prefix_pos = r.geom_part.REM; tp.prefix_len = r.geom_part.D0 + r.geom_part.D1; tp.pad = r.geom_part.pad;
-      unsigned long long* own = c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)nb + 1);
-      unsigned long long* cnt = r.gcnt.as<unsigned long long>();
+      unsigned long long* own_off = c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)nb + 1);
       const unsigned grid = (unsigned)((((first & 15) + nbb + POS_PER_THREAD - 1) / POS_PER_THREAD + NT - 1) / NT);
       GCU(cudaMemsetAsync(r.sizes32.p, 0, (size_t)nb * 4, c->stream));
       if (nbb) {
-        GCU(cudaMemsetAsync(d_out[i] + b0, 0xFF, nbb * 4, c->stream));
         k_occ_scatter<W, Elem, uint32_t, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, r.sizes32.as<uint32_t>(), nullptr,
-                                                                        nullptr, nullptr, 0, 0, cnt);
+                                                                        nullptr, nullptr, 0, 0, r.gcnt.as<unsigned long long>());
         c->launches++;
         GCU(cudaGetLastError());
       }
-      GCTX(c, scan_u32(c, r.sizes32.as<uint32_t>(), nb, own, nullptr));
+      GCTX(c, scan_u32(c, r.sizes32.as<uint32_t>(), nb, own_off, nullptr));
       if (nbb) {
-        GCU(cudaMemcpyAsync(c->occ_bcur.p, own, (size_t)nb * 8, cudaMemcpyDeviceToDevice, c->stream));
-        k_occ_scatter<W, Elem, uint32_t, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, nullptr, c->occ_bcur.as<unsigned long long>(),
-                                                                        c->B.as<Elem>(), r.gpos.as<uint32_t>(), 0, nbb, cnt);
-        c->launches++;
-        GCU(cudaGetLastError());
+        GCU(cudaMemcpyAsync(c->occ_bcur.p, own_off, (size_t)nb * 8, cudaMemcpyDeviceToDevice, c->stream));
+        int rc = place(i, b0, first, nbb, tp, grid);
+        if (rc) return rc;
       }
       if (i == 0) GCU(cudaEventRecord(r.gev[1], c->stream));
     }
     // -- every rank learns every rank's bucket sizes (this also orders the owners' reads after the senders' sweeps)
     { int rc = coll_allgather_dev(g, (size_t)g->rs[0].nb * 4, [&](int i) { return (const void*)g->rs[i].sizes32.p; },
                                   [&](int i) { return (void*)g->rs[i].sizes_all.p; }); if (rc) return rc; }
-    // -- owner: the pieces of its buckets, resolved in place in the senders' B
+    // -- owner: the pieces of its buckets in the senders' B
     for (int i = 0; i < nl; i++) {
       RankState& r = g->rs[i];
       apgk_ctx* c = r.c;
@@ -995,23 +1028,13 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
       FreqTable<W> ts = freq_table<W>(c);   // the shard's table, indexed by the finer bucket of the count (P + d2 bits)
       ts.nb = r.nbf; ts.prefix_pos = r.geom_shard.REM; ts.prefix_len = r.geom_shard.D0 + r.geom_shard.D1; ts.pad = r.geom_shard.pad;
       ts.D1 = r.geom_shard.D1;
-      GfArgs<Elem> a{};
-      a.src = (Elem* const*)r.ptrs_dev.p; a.piece_off = c->piece_off.as<unsigned long long>();
-      a.n_src = (uint32_t)world; a.nb = nb; a.me = (uint32_t)me;
-      a.d2 = r.geom_shard.D1 - r.geom_part.D1; a.rem_bits = r.geom_part.REM; a.pad = r.geom_part.pad;
-      a.counters = r.gcnt.as<unsigned long long>();
-      for (const auto& sg : g->own_segs) {
-        if ((int)sg[2] != me) continue;
-        a.lo = sg[0]; a.hi = sg[1];
-        k_gf_resolve<W, Elem, GF_NT><<<std::min<uint32_t>(sg[1] - sg[0], (uint32_t)c->n_sm * 8), GF_NT, 0, c->stream>>>(ts, a);
-        c->launches++;
-        GCU(cudaGetLastError());
-      }
+      int rc = own(i, ts);
+      if (rc) return rc;
     }
-    // -- all owners are done.  Their stores into this rank's B were made by kernels that had completed when their
-    // streams reached the barrier; a kernel's stores, peer stores included, are visible to every device once it has
-    // completed, and this rank's scatter runs after the barrier on its stream.  (The barrier also keeps the next
-    // batch's sweep from overwriting B while an owner still reads it.)
+    // -- all owners are done.  Their stores into this rank's B (the lookups write their answers there) were made by
+    // kernels that had completed when their streams reached the barrier; a kernel's stores, peer stores included,
+    // are visible to every device once it has completed, and what follows runs after the barrier on this rank's
+    // stream.  (The barrier also keeps the next batch's sweep from overwriting B while an owner still reads it.)
     { int rc = coll_barrier_dev(g); if (rc) return rc; }
     for (int i = 0; i < nl; i++) {
       RankState& r = g->rs[i];
@@ -1020,37 +1043,98 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
       GCU(cudaSetDevice(c->device));
       if (i == 0) GCU(cudaEventRecord(r.gev[2], c->stream));
       const uint64_t n = meta[me].n_bases, b0 = std::min(k * BB, n), nbb = std::min(BB, n - b0);
-      if (nbb) {
-        const unsigned long long* own = c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)r.nb + 1);
-        k_gf_scatter<Elem><<<(unsigned)std::min<uint64_t>((nbb + 255) / 256, (uint64_t)c->n_sm * 8), 256, 0, c->stream>>>(
-            c->B.as<Elem>(), r.gpos.as<uint32_t>(), own + r.nb, d_out[i] + b0, r.gcnt.as<unsigned long long>());
-        c->launches++;
-        GCU(cudaGetLastError());
-      }
+      int rc = after(i, b0, nbb);
+      if (rc) return rc;
       if (i == 0) GCU(cudaEventRecord(r.gev[3], c->stream));
     }
   }
-  // windows missing from their owner's table (or beyond their bucket) summed over the ranks: a table that does not
-  // match the reads fails the call on every rank
+  // the counters summed over the ranks: a table that does not match the reads fails the call on every rank
   { int rc = coll_allreduce_u64(g, 4, false, [&](int i) { return (const void*)g->rs[i].gcnt.p; },
                                 [&](int i) { return (void*)g->rs[i].red_out.p; }); if (rc) return rc; }
-  unsigned long long red[4] = {0, 0, 0, 0}, own[4] = {0, 0, 0, 0};
   GCU(cudaSetDevice(c0->device));
   GCU(cudaEventRecord(r0.gev[5], c0->stream));
   GCU(cudaMemcpyAsync(red, r0.red_out.p, 32, cudaMemcpyDeviceToHost, c0->stream));
-  GCU(cudaMemcpyAsync(own, r0.gcnt.p, 32, cudaMemcpyDeviceToHost, c0->stream));
+  GCU(cudaMemcpyAsync(own_cnt, r0.gcnt.p, 32, cudaMemcpyDeviceToHost, c0->stream));
   for (RankState& r : g->rs) { GCU(cudaSetDevice(r.c->device)); GCU(cudaStreamSynchronize(r.c->stream)); }
   if (n_batches) collect();
+  if (cudaEventElapsedTime(total_ms, r0.gev[4], r0.gev[5]) != cudaSuccess) *total_ms = 0;
+  return APGK_OK;
+}
+
+// the agreed batch size (the smallest over the ranks) and the number of batches (the largest)
+void exchange_plan(const std::vector<FreqMeta>& meta, uint64_t& BB, uint64_t& n_batches) {
+  BB = ~0ull; n_batches = 0;
+  for (const FreqMeta& m : meta) BB = std::min<uint64_t>(BB, m.batch_bases);
+  for (const FreqMeta& m : meta) n_batches = std::max<uint64_t>(n_batches, (m.n_bases + BB - 1) / BB);
+}
+
+template <int W, typename Elem>
+int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base, const std::vector<FreqMeta>& meta,
+                           apgk_group_freq_stats* st) {
+  const int world = g->world;
+  constexpr uint64_t eb = sizeof(Elem);
+  constexpr int NT = 128;
+  uint64_t BB, n_batches;
+  exchange_plan(meta, BB, n_batches);
+  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, false); };
+  auto start = [&](int) { return APGK_OK; };
+  // sender: every window's element into B bucket-major, its batch-relative position at the same slot of gpos
+  auto place = [&](int i, uint64_t b0, uint64_t first, uint64_t nbb, const FreqTable<W>& tp, unsigned grid) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    GCU(cudaMemsetAsync(d_out[i] + b0, 0xFF, nbb * 4, c->stream));
+    k_occ_scatter<W, Elem, uint32_t, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, nullptr, c->occ_bcur.as<unsigned long long>(),
+                                                                    c->B.as<Elem>(), r.gpos.as<uint32_t>(), 0, nbb, r.gcnt.as<unsigned long long>());
+    c->launches++;
+    GCU(cudaGetLastError());
+    return APGK_OK;
+  };
+  // owner: the pieces of its buckets resolved in place in the senders' B
+  auto own = [&](int i, const FreqTable<W>& ts) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    const int me = g->rank0 + i;
+    GfArgs<Elem> a{};
+    a.src = (Elem* const*)r.ptrs_dev.p; a.piece_off = c->piece_off.as<unsigned long long>();
+    a.n_src = (uint32_t)world; a.nb = r.nb; a.me = (uint32_t)me;
+    a.d2 = r.geom_shard.D1 - r.geom_part.D1; a.rem_bits = r.geom_part.REM; a.pad = r.geom_part.pad;
+    a.counters = r.gcnt.as<unsigned long long>();
+    for (const auto& sg : g->own_segs) {
+      if ((int)sg[2] != me) continue;
+      a.lo = sg[0]; a.hi = sg[1];
+      k_gf_resolve<W, Elem, GF_NT><<<std::min<uint32_t>(sg[1] - sg[0], (uint32_t)c->n_sm * 8), GF_NT, 0, c->stream>>>(ts, a);
+      c->launches++;
+      GCU(cudaGetLastError());
+    }
+    return APGK_OK;
+  };
+  // sender: the answers to their positions
+  auto after = [&](int i, uint64_t b0, uint64_t nbb) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    const int me = g->rank0 + i;
+    if (nbb) {
+      const unsigned long long* own_off = c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)r.nb + 1);
+      k_gf_scatter<Elem><<<(unsigned)std::min<uint64_t>((nbb + 255) / 256, (uint64_t)c->n_sm * 8), 256, 0, c->stream>>>(
+          c->B.as<Elem>(), r.gpos.as<uint32_t>(), own_off + r.nb, d_out[i] + b0, r.gcnt.as<unsigned long long>());
+      c->launches++;
+      GCU(cudaGetLastError());
+    }
+    return APGK_OK;
+  };
+  unsigned long long red[4] = {0, 0, 0, 0}, cnt[4] = {0, 0, 0, 0};
+  float ms[3], total = 0;
+  { int rc = exchange_batches<W, Elem>(g, meta, first_base, BB, n_batches, need_B, start, place, own, after, red, cnt, ms, &total); if (rc) return rc; }
   if (red[0] || red[2])
     GFAIL(APGK_E_STATE, "group read_freqs: %llu windows missing from their owner's table, %llu beyond their bucket (the tables do not match the reads)",
           red[0], red[2]);
   if (st) {
     *st = apgk_group_freq_stats{};
     st->n_batches = (int32_t)n_batches;
-    st->n_queries = own[3];
-    st->remote_bytes = own[1] * (eb + 4);
+    st->n_queries = cnt[3];
+    st->remote_bytes = cnt[1] * (eb + 4);
     st->sweep_ms = ms[0]; st->exchange_ms = ms[1]; st->scatter_ms = ms[2];
-    cudaEventElapsedTime(&st->total_ms, r0.gev[4], r0.gev[5]);
+    st->total_ms = total;
   }
   return APGK_OK;
 }
@@ -1076,6 +1160,130 @@ int group_read_freqs(apgk_group* g, uint32_t* const* d_out, const uint64_t* firs
   if (c0->W == 1) return group_read_freqs_typed<1, Key<1>>(g, d_out, first_base, meta, st);
   if (c0->W == 2) return group_read_freqs_typed<2, Key<2>>(g, d_out, first_base, meta, st);
   return group_read_freqs_typed<3, Key<3>>(g, d_out, first_base, meta, st);
+}
+
+// ---------------------------------------------------------------- affixes on the sharded table
+// apgk_group_build_affixes; the kernels and the data flow are described in gaffix.cuh.
+
+int gaff_prepare(apgk_group* g, int i, FreqMeta& m) {
+  RankState& r = g->rs[i];
+  apgk_ctx* c = r.c;
+  const int me = g->rank0 + i;
+  m = FreqMeta{};
+  m.cap_B = c->B.cap; m.cap_sub = c->sub_sizes.cap;
+  m.ptr_B = (uint64_t)(uintptr_t)c->B.p; m.ptr_sub = (uint64_t)(uintptr_t)c->sub_sizes.p;
+  if (!g->counted || !g->freq_ready)
+    GFAIL(APGK_E_STATE, "apgk_group_build_affixes needs a completed apgk_group_count with APGK_WANT_COUNTS");
+  if (c->gen != r.gen_counted)
+    GFAIL(APGK_E_STATE, "rank %d: its context was reset, given reads or counted on its own since apgk_group_count: count again", me);
+  m.n_bases = c->total_bases;
+  GCU(cudaSetDevice(c->device));
+  exchange_batch(g, i, m);
+  GCU(c->aff.ensure(((c->n_distinct + 3) & ~3ull) + 4));
+  return exchange_buffers(g, i, true, m);
+}
+
+template <int W, typename Elem>
+int group_build_affixes_typed(apgk_group* g, const std::vector<FreqMeta>& meta, apgk_group_affix_stats* st) {
+  const int world = g->world;
+  constexpr uint64_t eb = sizeof(Elem);
+  constexpr bool U32 = eb == 4;
+  constexpr int NT = 128;
+  uint64_t BB, n_batches;
+  exchange_plan(meta, BB, n_batches);
+  // the byte planes' offsets in the senders' B follow from the all-gathered sizes: every owner knows them unasked
+  std::vector<uint64_t> plane(world), first_base(g->n_local, 0);
+  for (int s = 0; s < world; s++) plane[s] = aff_plane(std::min(BB, meta[s].n_bases), eb);
+  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, true); };
+  for (RankState& r : g->rs) { r.c->have_aff = false; r.c->aff_group = false; }
+  // the plane offsets beside the peers' pointers; the affix array zeroed (timed with the call: part of its cost)
+  auto start = [&](int i) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    GCU(cudaMemcpyAsync(r.ptrs_dev.as<unsigned char>() + (size_t)world * 8, plane.data(), (size_t)world * 8, cudaMemcpyHostToDevice, c->stream));
+    GCU(cudaMemsetAsync(c->aff.p, 0, ((c->n_distinct + 3) & ~3ull) + 4, c->stream));
+    return APGK_OK;
+  };
+  // sender: every window's element and affix byte into B bucket-major; counters[3] += the windows placed
+  auto place = [&](int i, uint64_t, uint64_t first, uint64_t nbb, const FreqTable<W>& tp, unsigned grid) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    const int me = g->rank0 + i;
+    unsigned long long* cnt = r.gcnt.as<unsigned long long>();
+    unsigned long long* elem64 = U32 ? c->B.as<unsigned long long>() : nullptr;
+    Key<W>* keys = U32 ? nullptr : c->B.as<Key<W>>();
+    uint8_t* bytes = U32 ? nullptr : c->B.as<uint8_t>() + plane[me];
+    k_aff_scatter<W, Elem, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, c->occ_bcur.as<unsigned long long>(), elem64,
+                                                          keys, bytes, nbb, cnt);
+    c->launches++;
+    GCU(cudaGetLastError());
+    k_gaff_sent<<<1, 1, 0, c->stream>>>(c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)r.nb + 1) + r.nb, cnt);
+    c->launches++;
+    GCU(cudaGetLastError());
+    return APGK_OK;
+  };
+  // owner: the pieces of its buckets read from the senders' B and ORed into its own rows
+  auto own = [&](int i, const FreqTable<W>& ts) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    const int me = g->rank0 + i;
+    GaffArgs a{};
+    a.src = (const void* const*)r.ptrs_dev.p;
+    a.plane_off = r.ptrs_dev.as<unsigned long long>() + world;
+    a.piece_off = c->piece_off.as<unsigned long long>();
+    a.n_src = (uint32_t)world; a.nb = r.nb; a.me = (uint32_t)me;
+    a.d2 = r.geom_shard.D1 - r.geom_part.D1; a.rem_bits = r.geom_part.REM; a.pad = r.geom_part.pad;
+    a.aff32 = c->aff.as<uint32_t>();
+    a.counters = r.gcnt.as<unsigned long long>();
+    for (const auto& sg : g->own_segs) {
+      if ((int)sg[2] != me) continue;
+      a.lo = sg[0]; a.hi = sg[1];
+      k_gaff_place<W, Elem, GF_NT><<<std::min<uint32_t>(sg[1] - sg[0], (uint32_t)c->n_sm * 8), GF_NT, 0, c->stream>>>(ts, a);
+      c->launches++;
+      GCU(cudaGetLastError());
+    }
+    return APGK_OK;
+  };
+  auto after = [&](int, uint64_t, uint64_t) { return APGK_OK; };   // nothing comes back to the sender
+  unsigned long long red[4] = {0, 0, 0, 0}, cnt[4] = {0, 0, 0, 0};
+  float ms[3], total = 0;
+  { int rc = exchange_batches<W, Elem>(g, meta, first_base.data(), BB, n_batches, need_B, start, place, own, after, red, cnt, ms, &total); if (rc) return rc; }
+  if (red[0] || red[2])
+    GFAIL(APGK_E_STATE, "group affixes: %llu windows missing from their owner's table, %llu beyond their bucket (the tables do not match the reads)",
+          red[0], red[2]);
+  for (RankState& r : g->rs) { r.c->have_aff = true; r.c->aff_group = true; }
+  if (st) {
+    *st = apgk_group_affix_stats{};
+    st->n_batches = (int32_t)n_batches;
+    st->n_windows = cnt[3];
+    st->remote_bytes = cnt[1] * (U32 ? 8 : eb + 1);
+    st->sweep_ms = ms[0]; st->exchange_ms = ms[1];
+    st->total_ms = total;
+  }
+  return APGK_OK;
+}
+
+int group_build_affixes(apgk_group* g, apgk_group_affix_stats* st) {
+  if (g->dead) GFAIL(APGK_E_STATE, "a context of this group has been destroyed");
+  const int world = g->world, nl = g->n_local;
+  std::vector<FreqMeta> mine(nl), meta(world);
+  std::string own_err;
+  for (int i = 0; i < nl; i++) {
+    const int rc = gaff_prepare(g, i, mine[i]);
+    if (rc) { mine[i].status = rc; if (own_err.empty()) own_err = g->err; }
+  }
+  { int rc = coll_allgather_host(g, mine.data(), sizeof(FreqMeta), meta.data()); if (rc) return rc; }
+  for (int s = 0; s < world; s++)
+    if (meta[s].status) {
+      if (own_err.empty()) GFAIL(meta[s].status, "rank %d refused the affix build (error %d; its apgk_group_last_error says why)", s, meta[s].status);
+      g->err = own_err;
+      return meta[s].status;
+    }
+  apgk_ctx* c0 = g->rs[0].c;
+  if (c0->elem_bytes == 4) return group_build_affixes_typed<1, uint32_t>(g, meta, st);
+  if (c0->W == 1) return group_build_affixes_typed<1, Key<1>>(g, meta, st);
+  if (c0->W == 2) return group_build_affixes_typed<2, Key<2>>(g, meta, st);
+  return group_build_affixes_typed<3, Key<3>>(g, meta, st);
 }
 
 }  // namespace

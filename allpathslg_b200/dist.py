@@ -95,6 +95,17 @@ def sharded_read_freqs(kc, rank, world, first_base=0, n_bases=None, group=None, 
     return grp.read_freqs([first_base], None if n_bases is None else [n_bases], stats=stats)[0]
 
 
+def sharded_affixes(kc, rank, world, group=None, stats=None):
+    """After `sharded_count`: the affix byte of every row of this rank's shard table (the rows of `kc.counts()`),
+    taken over ALL ranks' reads, as a host uint8 array.  Collective: every rank calls it
+    (apgk_group_build_affixes).  The bytes stay in `kc` for kc.affixes() / kc.lookup_affixes()."""
+    grp = _group_of(kc, rank, world, group)
+    st = grp.build_affixes()
+    if stats is not None:
+        stats.update(st)
+    return kc.affixes()
+
+
 def _group_of(kc, rank, world, group=None):
     """The library-side group of this counter (made once: rank 0's id is broadcast over torch.distributed)."""
     from .kmers import KmerGroup

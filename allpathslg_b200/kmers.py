@@ -486,6 +486,14 @@ class KmerGroup:
             stats.update(st)
         return [b.cpu().numpy().view(np.uint32)[: int(n)] for b, n in zip(bufs, n_bases)]
 
+    def build_affixes(self):
+        """K-mer affixes on the sharded table (collective): afterwards every local counter's affixes() /
+        lookup_affixes() answer for the k-mers its shard owns, each byte taken over all ranks' reads.
+        -> dict(n_batches, n_windows, remote_bytes, sweep_ms, exchange_ms, total_ms)."""
+        st = _lib.GroupAffixStats()
+        self._ck(self._L.apgk_group_build_affixes(self._h, C.byref(st)))
+        return {k: getattr(st, k) for k, _ in st._fields_}
+
     def _ranges(self, first_base, n_bases):
         n = len(self.counters)
         if first_base is None:

@@ -195,7 +195,8 @@ int apgk_occurrences_copy(apgk_ctx* ctx, uint64_t first_kmer, uint64_t n_kmers, 
  * Encoding: one byte per distinct k-mer, row i of the sorted table (apgk_counts_copy row i); bit b (0..3) = base b
  * (A, C, G, T) precedes c, bit 4+b = base b follows c.
  * apgk_build_affixes needs a context finished by apgk_finish with APGK_WANT_COUNTS, its read store in place (the same
- * precondition as apgk_build_occurrences): APGK_E_STATE otherwise, also on a shard after apgk_group_count and after
+ * precondition as apgk_build_occurrences): APGK_E_STATE otherwise, also on a shard after apgk_group_count (a shard's
+ * affixes come from apgk_group_build_affixes) and after
  * apgk_finish_keys_device / apgk_count_pieces*; APGK_E_RANGE when a count saturated.  ms3 (may be NULL) = device
  * milliseconds of {clear + run-offset scan, sweep of the reads, per-bucket OR}.  The affixes live in a buffer of their
  * own: they survive apgk_release_temp, apgk_build_occurrences and apgk_read_freqs*, and are dropped by whatever
@@ -354,6 +355,27 @@ typedef struct {
 } apgk_group_freq_stats;
 int apgk_group_read_freqs_device(apgk_group* g, uint32_t* const* d_out, const uint64_t* first_base,
                                  const uint64_t* n_bases, apgk_group_freq_stats* stats);
+/* K-mer affixes on the sharded table: apgk_build_affixes for a group.  After apgk_group_count with APGK_WANT_COUNTS,
+ * every local context holds, for each row of its shard table, the affix byte of that k-mer taken over ALL ranks'
+ * reads, with the definition and encoding of apgk_build_affixes (palindromes included).  Every window's level-1
+ * element and affix byte travel to the k-mer's owner on the query exchange of apgk_group_read_freqs_device (per
+ * batch of the rank's whole read store; every rank runs the same number of batches); the owner reads the pieces of
+ * its buckets over peer memory and ORs the bytes into its own rows.  Nothing is written to a peer.
+ * Afterwards apgk_affixes_device / apgk_affixes_copy / apgk_lookup_affixes answer on each shard for the k-mers it
+ * owns; a k-mer it does not own gives (0, 0), as an absent one.  The affixes survive apgk_release_temp and
+ * apgk_group_read_freqs_device, and are dropped by whatever drops the shard table (apgk_group_count, apgk_add_reads*,
+ * apgk_finish*, apgk_reset).  apgk_build_affixes on a shard still refuses with APGK_E_STATE.
+ * Collective; stats may be NULL.  Errors come back identical on every rank: APGK_E_STATE without a current count with
+ * APGK_WANT_COUNTS, when a member context was reset, given reads or counted on its own since (apgk_release_temp is
+ * fine), or when a window's k-mer is missing from its owner's table (the affixes are then not built on any rank);
+ * APGK_E_NOMEM when a rank's buffers do not fit. */
+typedef struct {
+  int32_t n_batches;        /* exchange batches this call ran (agreed by all ranks) */
+  uint64_t n_windows;       /* valid windows of this rank's read store that were sent */
+  uint64_t remote_bytes;    /* bytes this rank's owner-side kernel read from peers' memory */
+  float sweep_ms, exchange_ms, total_ms;   /* device time, first local context */
+} apgk_group_affix_stats;
+int apgk_group_build_affixes(apgk_group* g, apgk_group_affix_stats* stats);
 
 /* ---- instrumentation */
 #define APGK_N_STAGES 14

@@ -2,7 +2,8 @@
 collectives, CUDA IPC peer memory for the exchange) on real GPUs, against the oracle on the union of all ranks' reads.
 Single-round cases and k-mer-space rounds (outer + inner), several K, a second step on the same group; after each
 step every rank's frequency lookups on the sharded table (apgk_group_read_freqs_device) for every window of its reads,
-against the oracle's global table applied to them.
+against the oracle's global table applied to them, and every rank's affixes (apgk_group_build_affixes) for the rows
+of its shard, against the affix oracle over all ranks' reads.
 
    python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port 29511 tools/dist_check.py
 """
@@ -10,12 +11,14 @@ import os
 import sys
 
 sys.path.insert(0, ".")
+sys.path.insert(0, "tests")
 import numpy as np
 import torch
 import torch.distributed as dist
 
 from allpathslg_b200 import KmerCounter, synth_params
-from allpathslg_b200.dist import sharded_count, sharded_read_freqs
+import affix_oracle as AO
+from allpathslg_b200.dist import sharded_affixes, sharded_count, sharded_read_freqs
 from oracle import oracle_a as A
 
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
@@ -47,6 +50,7 @@ for (K, G, L, n_per, rounds) in CASES:
     pr, orr = A.synth_reads(A.synth_params(G, L), rank * n_per, n_per)
     erf = A.read_freqs(pr, orr, K, ek, ec)
     erf = np.where(erf == np.uint64(0xFFFFFFFFFFFFFFFF), np.uint64(0xFFFFFFFF), erf).astype(np.uint32)
+    eaff = AO.affixes_a(packed, off, K, ek)
     for step in range(2):
         tm = {}
         spec, ni, nd = sharded_count(kc, rank, world, timings=tm)
@@ -54,15 +58,19 @@ for (K, G, L, n_per, rounds) in CASES:
         good = ni == en and nd == len(ek) and len(spec) == len(es) and bool((spec == es).all())
         good = good and (tm["n_rounds"] >= rounds[1] if rounds else tm["n_rounds"] == 1)
         hits = np.zeros(len(ek), dtype=np.int64)
+        afs = {}
+        gaff = sharded_affixes(kc, rank, world, stats=afs)
+        aff_ok = len(gaff) == len(gk)
         if len(gk):
             idx = np.searchsorted(er, rows(gk))
             good = good and bool((idx < len(er)).all())
             idx = np.minimum(idx, len(er) - 1)
             good = good and bool((er[idx] == rows(gk)).all()) and bool((ec[idx] == gc.astype(np.uint64)).all()) and bool((np.diff(idx) > 0).all())
             hits[idx] += 1
+            aff_ok = aff_ok and bool((gaff == eaff[idx]).all())
         fst = {}
         freqs_ok = bool((sharded_read_freqs(kc, rank, world, stats=fst) == erf).all())
-        good = good and freqs_ok
+        good = good and freqs_ok and aff_ok
         t = torch.from_numpy(hits).cuda()
         dist.all_reduce(t)
         good = good and bool((t == 1).all().item())   # every k-mer of the oracle sits in exactly one shard
@@ -70,10 +78,12 @@ for (K, G, L, n_per, rounds) in CASES:
         dist.all_reduce(f, op=dist.ReduceOp.MIN)
         if rank == 0:
             print("K=%d world=%d step=%d instances=%d distinct=%d all-ranks-ok=%s  (%s, rounds %d/%d, P=%d+%d; rank0: shard %d, "
-                  "remote %.1f MB in %.3f ms = %.1f GB/s, step %.2f ms; read-freqs rank0 %s, %.1f MB remote, %.2f ms)" %
+                  "remote %.1f MB in %.3f ms = %.1f GB/s, step %.2f ms; read-freqs rank0 %s, %.1f MB remote, %.2f ms; "
+                  "affixes rank0 %s, %.1f MB remote, %.2f ms)" %
                   (K, world, step, ni, nd, bool(f.item()), tm["path"], tm["n_outer_rounds"], tm["n_rounds"], tm["prefix_bits"],
                    tm["split_bits"], tm["shard_instances"], tm["remote_bytes"] / 1e6, tm["gather_ms"], tm["gather_remote_GBps"],
-                   tm["step_ms"], freqs_ok, fst["remote_bytes"] / 1e6, fst["total_ms"]), flush=True)
+                   tm["step_ms"], freqs_ok, fst["remote_bytes"] / 1e6, fst["total_ms"], aff_ok, afs["remote_bytes"] / 1e6,
+                   afs["total_ms"]), flush=True)
         ok = ok and bool(f.item())
     kc._group.close()
     dist.barrier()   # every rank has unmapped the peers' buffers before anyone frees its own
