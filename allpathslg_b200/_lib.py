@@ -38,6 +38,12 @@ class GroupAffixStats(C.Structure):
                 ("exchange_ms", C.c_float), ("total_ms", C.c_float)]
 
 
+class GroupOccStats(C.Structure):
+    _fields_ = [("n_batches", C.c_int32), ("n_windows", C.c_uint64), ("n_occ", C.c_uint64), ("n_big_runs", C.c_uint64),
+                ("remote_bytes", C.c_uint64), ("sweep_ms", C.c_float), ("exchange_ms", C.c_float), ("sort_ms", C.c_float),
+                ("total_ms", C.c_float)]
+
+
 class SynthParams(C.Structure):
     _fields_ = [("genome_len", C.c_uint64), ("seed_g", C.c_uint64), ("seed_p", C.c_uint64), ("seed_q", C.c_uint64),
                 ("seed_r", C.c_uint64), ("seed_e", C.c_uint64), ("read_len", C.c_uint32), ("err_per_200", C.c_uint32)]
@@ -107,6 +113,7 @@ SYMBOLS = {
     "apgk_group_stats_get": (C.c_int, [_vp, C.POINTER(GroupStats)]),
     "apgk_group_read_freqs_device": (C.c_int, [_vp, _vp, _vp, _vp, C.POINTER(GroupFreqStats)]),
     "apgk_group_build_affixes": (C.c_int, [_vp, C.POINTER(GroupAffixStats)]),
+    "apgk_group_build_occurrences": (C.c_int, [_vp, C.POINTER(GroupOccStats)]),
     "apgk_spectrum_device": (C.c_int, [_vp, C.POINTER(_vp), _u64p]),
     "apgk_spectrum_reload": (C.c_int, [_vp]),
     "apgk_stage_ms": (C.c_int, [_vp, C.POINTER(C.c_float)]),

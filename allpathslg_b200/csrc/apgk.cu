@@ -22,6 +22,7 @@
 #include "gfreq.cuh"
 #include "affix.cuh"
 #include "gaffix.cuh"
+#include "gocc.cuh"
 
 using namespace apgk;
 
@@ -80,6 +81,7 @@ struct apgk_ctx {
   // ---- read store
   DevBuf bases, starts, staging, off_dev;
   uint64_t total_bases = 0, n_reads = 0;
+  uint64_t max_read_len = 0;         // longest read added (group occurrence records keep a position in 31 bits)
   uint64_t n_windows = 0;            // exact k-mer instances of the store: sum over reads of max(0, L - K + 1)
   uint64_t n_windows_run = 0;        // instances the current step's level-0 histogram must find (store, or a key array)
   // ---- streamed ingest (APGK_ASYNC_INGEST): copies in flight on copy_stream, one event per slice
@@ -105,7 +107,9 @@ struct apgk_ctx {
   bool table_from_reads = false;   // the table counts exactly the windows of this context's read store
   // ---- occurrence records (apgk_build_occurrences): run offsets + (position << 1 | rc) per instance, in A
   DevBuf occ, occ_pos, occ_off, occ_cnt, occ_bstart, occ_bcur, rank_cnt, rank_dir, empty_dev, occ_tmp;
+  DevBuf occ_cur, occ_big;         // group build (gocc.cuh): per-row cursors, big-run list
   bool have_occ = false;
+  bool occ_group = false;          // the records of a shard, built by apgk_group_build_occurrences (read-id encoding)
   uint64_t n_occ = 0, n_big_runs = 0;
   float occ_ms[5]{};
   float freq_ms[3]{};              // last bulk read_freqs: {memset + scan, sweep, placement}
@@ -388,7 +392,7 @@ int append_bases(apgk_ctx* c, const uint8_t* packed, uint64_t first_base, uint64
 
 void invalidate_results(apgk_ctx* c) {
   c->finished = false; c->have_table = false; c->spec_loaded = false;
-  c->table_from_reads = false; c->have_occ = false; c->n_occ = 0;
+  c->table_from_reads = false; c->have_occ = false; c->occ_group = false; c->n_occ = 0;
   c->have_aff = false; c->aff_group = false;
   c->n_instances = c->n_distinct = 0;
   c->owner_ranks = 0;
@@ -1269,7 +1273,7 @@ int occ_scatter_phase(apgk_ctx* c, unsigned long long* counters, OccScatter& o) 
 template <int W, typename Elem>
 int build_occurrences_impl(apgk_ctx* c) {
   const uint64_t N = c->n_instances, D = c->n_distinct;
-  c->have_occ = false; c->n_occ = 0; c->n_big_runs = 0;
+  c->have_occ = false; c->occ_group = false; c->n_occ = 0; c->n_big_runs = 0;
   for (float& m : c->occ_ms) m = 0;
   { int rc = wait_ingest(c); if (rc) return rc; }
   for (cudaEvent_t& e : c->occ_ev) if (!e) CU(cudaEventCreate(&e));
@@ -1492,9 +1496,12 @@ int occurrences_copy_impl(apgk_ctx* c, uint64_t first, uint64_t n_kmers, uint64_
   for (uint64_t done = 0; done < n; done += CH) {
     const uint64_t m = std::min(CH, n - done);
     int32_t* d_pos = (int32_t*)(d_id + m);
-    k_occ_translate<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(
-        c->occ.as<unsigned long long>() + o0 + done, m, c->starts.as<uint32_t>(), c->rank_dir.as<unsigned long long>(),
-        c->empty_dev.as<unsigned long long>(), (uint32_t)c->empty_nb.size(), d_id, d_pos);
+    if (c->occ_group)   // a shard's records already carry the group read id
+      k_gocc_decode<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(c->occ.as<unsigned long long>() + o0 + done, m, d_id, d_pos);
+    else
+      k_occ_translate<<<(unsigned)((m + 255) / 256), 256, 0, c->stream>>>(
+          c->occ.as<unsigned long long>() + o0 + done, m, c->starts.as<uint32_t>(), c->rank_dir.as<unsigned long long>(),
+          c->empty_dev.as<unsigned long long>(), (uint32_t)c->empty_nb.size(), d_id, d_pos);
     LAUNCHED();
     if (read_id_out) CU(cudaMemcpyAsync(read_id_out + done, d_id, m * 4, cudaMemcpyDeviceToHost, c->stream));
     if (pos_out) CU(cudaMemcpyAsync(pos_out + done, d_pos, m * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -1777,7 +1784,7 @@ void apgk_destroy(apgk_ctx* c) {
                    &c->big_list, &c->stats, &c->scratch, &c->stacks, &c->spec_dense, &c->spec_ovf, &c->misc, &c->deferred,
                    &c->out_keys, &c->out_cnt, &c->owner_plan_dev, &c->piece_off, &c->piece_tmp, &c->piece_ptrs, &c->C2, &c->sub_sizes, &c->TK,
                    &c->occ, &c->occ_pos, &c->occ_off, &c->occ_cnt, &c->occ_bstart, &c->occ_bcur, &c->rank_cnt, &c->rank_dir, &c->empty_dev,
-                   &c->occ_tmp, &c->aff};
+                   &c->occ_tmp, &c->aff, &c->occ_cur, &c->occ_big};
   for (DevBuf* b : all) b->release();
   for (cudaEvent_t e : c->occ_ev) if (e) cudaEventDestroy(e);
   for (auto& iv : c->ivs) { cudaEventDestroy(iv.e0); cudaEventDestroy(iv.e1); }
@@ -1800,7 +1807,7 @@ int apgk_reset(apgk_ctx* c) {
     CU(cudaMemsetAsync(c->bases.p, 0, std::min(c->bases.cap, (size_t)((c->total_bases + 31) / 32) * 8 + 256), c->stream));
     CU(cudaMemsetAsync(c->starts.p, 0, std::min(c->starts.cap, (size_t)((c->total_bases + 31) / 32) * 4 + 256), c->stream));
   }
-  c->total_bases = 0; c->n_reads = 0; c->n_windows = 0;
+  c->total_bases = 0; c->n_reads = 0; c->n_windows = 0; c->max_read_len = 0;
   c->empty_nb.clear();
   invalidate_results(c);
   return APGK_OK;
@@ -1829,6 +1836,7 @@ int apgk_add_reads(apgk_ctx* c, const uint8_t* packed, const uint64_t* off, uint
   for (uint64_t r = 0; r < n_reads; r++) {  // reads without bases own no start bit: remember where they sit (occurrence read ids)
     const uint64_t len = off[r + 1] - off[r];
     if (len == 0) c->empty_nb.push_back(c->n_reads + r - c->empty_nb.size());
+    c->max_read_len = std::max(c->max_read_len, len);
     if (len >= (uint64_t)c->cfg.K) c->n_windows += len - (uint64_t)c->cfg.K + 1;
   }
   c->total_bases += nb; c->n_reads += n_reads;
@@ -1872,6 +1880,7 @@ int apgk_add_reads_uniform(apgk_ctx* c, const uint8_t* packed, uint64_t first_ba
                                                                                    c->starts.as<uint32_t>());
     LAUNCHED();
     c->total_bases += nb; c->n_reads += n_reads;
+    c->max_read_len = std::max<uint64_t>(c->max_read_len, read_len);
     if (read_len >= (uint32_t)c->cfg.K) c->n_windows += n_reads * (uint64_t)(read_len - (uint32_t)c->cfg.K + 1);
     invalidate_results(c);
     c->n_slices = n_sl;
@@ -1885,6 +1894,7 @@ int apgk_add_reads_uniform(apgk_ctx* c, const uint8_t* packed, uint64_t first_ba
   LAUNCHED();
   CU(cudaStreamSynchronize(c->stream));
   c->total_bases += nb; c->n_reads += n_reads;
+  c->max_read_len = std::max<uint64_t>(c->max_read_len, read_len);
   if (read_len >= (uint32_t)c->cfg.K) c->n_windows += n_reads * (uint64_t)(read_len - (uint32_t)c->cfg.K + 1);
   invalidate_results(c);
   return APGK_OK;
@@ -1910,6 +1920,7 @@ int apgk_synth_reads(apgk_ctx* c, const apgk_synth_params* p, uint64_t r0, uint6
   LAUNCHED();
   CU(cudaStreamSynchronize(c->stream));
   c->total_bases += nb; c->n_reads += n_reads;
+  c->max_read_len = std::max<uint64_t>(c->max_read_len, p->read_len);
   if (p->read_len >= (uint32_t)c->cfg.K) c->n_windows += n_reads * (uint64_t)(p->read_len - (uint32_t)c->cfg.K + 1);
   invalidate_results(c);
   return APGK_OK;
@@ -2165,10 +2176,10 @@ int apgk_release_temp(apgk_ctx* c) {
   CU(cudaStreamSynchronize(c->stream));
   // B and sub_sizes stay: the peers of a group may have them mapped
   DevBuf* tmp[] = {&c->A, &c->T, &c->C2, &c->TK, &c->scratch, &c->stacks, &c->chunksum, &c->chunksum0, &c->piece_off, &c->piece_tmp,
-                   &c->occ, &c->occ_pos, &c->occ_tmp, &c->staging};
+                   &c->occ, &c->occ_pos, &c->occ_tmp, &c->staging, &c->occ_cur, &c->occ_big};
   for (DevBuf* b : tmp) b->release();
   c->hp0_elems = ~0ull;            // the level-0 plan's chunk rows went with chunksum0
-  c->have_occ = false; c->n_occ = 0;
+  c->have_occ = false; c->occ_group = false; c->n_occ = 0;
   c->part_ready = false; c->part_n = 0;
   c->tmp_keys_last = nullptr;
   return APGK_OK;
@@ -2268,7 +2279,7 @@ int apgk_occurrences_info(const apgk_ctx* c, uint64_t* n_occ, uint64_t* n_big_ru
 
 int apgk_occurrences_device(apgk_ctx* c, const uint64_t** d_run_off, const uint64_t** d_occ, uint64_t* n_occ) {
   if (!c) return APGK_E_ARG;
-  if (!c->have_occ) FAIL(APGK_E_STATE, "no occurrences: call apgk_build_occurrences first");
+  if (!c->have_occ) FAIL(APGK_E_STATE, "no occurrences: call apgk_build_occurrences (apgk_group_build_occurrences on a shard) first");
   if (d_run_off) *d_run_off = c->occ_off.as<uint64_t>();
   if (d_occ) *d_occ = c->n_occ ? c->occ.as<uint64_t>() : nullptr;
   if (n_occ) *n_occ = c->n_occ;
@@ -2278,7 +2289,7 @@ int apgk_occurrences_device(apgk_ctx* c, const uint64_t** d_run_off, const uint6
 int apgk_occurrences_copy(apgk_ctx* c, uint64_t first_kmer, uint64_t n_kmers, uint64_t* run_off_out, uint32_t* read_id_out,
                           int32_t* pos_out) {
   if (!c) return APGK_E_ARG;
-  if (!c->have_occ) FAIL(APGK_E_STATE, "no occurrences: call apgk_build_occurrences first");
+  if (!c->have_occ) FAIL(APGK_E_STATE, "no occurrences: call apgk_build_occurrences (apgk_group_build_occurrences on a shard) first");
   if (first_kmer > c->n_distinct || n_kmers > c->n_distinct - first_kmer) FAIL(APGK_E_ARG, "k-mer range beyond the table");
   CU(cudaSetDevice(c->device));
   return occurrences_copy_impl(c, first_kmer, n_kmers, run_off_out, read_id_out, pos_out);
@@ -2576,6 +2587,11 @@ int apgk_group_read_freqs_device(apgk_group* g, uint32_t* const* d_out, const ui
 int apgk_group_build_affixes(apgk_group* g, apgk_group_affix_stats* stats) {
   if (!g) return APGK_E_ARG;
   return group_build_affixes(g, stats);
+}
+
+int apgk_group_build_occurrences(apgk_group* g, apgk_group_occ_stats* stats) {
+  if (!g) return APGK_E_ARG;
+  return group_build_occurrences(g, stats);
 }
 
 int apgk_group_totals(const apgk_group* g, uint64_t* n_instances, uint64_t* n_distinct) {

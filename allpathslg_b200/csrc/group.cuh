@@ -853,32 +853,42 @@ int group_count(apgk_group* g) {
 // ---------------------------------------------------------------- frequency lookups on the sharded table
 // apgk_group_read_freqs_device; the kernels and the data flow are described in gfreq.cuh.
 
-struct FreqMeta {   // what every rank tells the others before a lookup or an affix build (all-gathered, host side)
+struct FreqMeta {   // what every rank tells the others before an exchange over the read stores (all-gathered, host side)
   int32_t status, pad_;   // 0, or the error this rank met while preparing
   uint64_t n_bases, batch_bases, cap_B, cap_sub, ptr_B, ptr_sub;
+  uint64_t n_reads;       // the occurrence build: reads of the rank's store (group read ids follow from them)
 };
 
-// Bytes of B one batch of n bases takes: the level-1 elements (eb bytes), and for the affix build (gaffix.cuh) their
-// affix bytes -- one u64 per slot with a 4-byte remainder, else a byte plane behind the keys at a 16-byte aligned
-// offset (aff_plane), inside the same exported buffer.
-uint64_t aff_plane(uint64_t n, uint64_t eb) { return eb == 4 ? 0 : (n * eb + 15) & ~15ull; }
-uint64_t exchange_B_bytes(uint64_t n, uint64_t eb, bool aff) { return (!aff ? n * eb : eb == 4 ? n * 8 : aff_plane(n, eb) + n) + 16; }
+// What travels beside the level-1 elements of an exchange: nothing for the lookups (the answers are written over
+// the elements), the affix byte (gaffix.cuh), or the occurrence record (gocc.cuh).
+enum Payload { PL_FREQ, PL_AFF, PL_OCC };
 
-// The preparation the exchanges over a rank's read store share (the lookups and the affix build), in two steps around
-// the caller's own allocations (the lookups' positions, the affix array), so that the check whether B can grow sees
-// the memory those took.  exchange_batch: the batch size from the budget of the count's temp buffers -- per base at
-// most one element in B and 4 more bytes (the lookups' position; the affix byte, or the u64 slot of a 4-byte
-// remainder, fits in them).  exchange_buffers: the buffers of a batch, then whether B can grow to hold one.  It must
-// come after every other allocation of the preparation: B grows later, after a collective, where a rank that failed
-// alone would leave the others waiting.
-void exchange_batch(apgk_group* g, int i, FreqMeta& m) {
+// Bytes of B one batch of n bases takes: the level-1 elements (eb bytes) at offset 0, then the payload inside the
+// same exported buffer.  Affixes: one u64 per slot with a 4-byte remainder (rem << 8 | affix), else a byte plane
+// behind the keys; records: a u64 plane behind the elements.  A plane starts at a 16-byte aligned offset
+// (payload_plane) that every rank derives from the all-gathered sizes.
+uint64_t payload_plane(uint64_t n, uint64_t eb, Payload pl) { return pl == PL_AFF && eb == 4 ? 0 : (n * eb + 15) & ~15ull; }
+uint64_t exchange_B_bytes(uint64_t n, uint64_t eb, Payload pl) {
+  if (pl == PL_FREQ) return n * eb + 16;
+  if (pl == PL_AFF) return (eb == 4 ? n * 8 : payload_plane(n, eb, pl) + n) + 16;
+  return payload_plane(n, eb, pl) + n * 8 + 16;
+}
+
+// The preparation the exchanges over a rank's read store share (the lookups, the affix and the occurrence builds), in
+// two steps around the caller's own allocations (the lookups' positions, the affix array, the records), so that the
+// check whether B can grow sees the memory those took.  exchange_batch: the batch size from the budget of the count's
+// temp buffers -- per base at most one element in B and payload_bytes more (4 for the lookups' position and for the
+// affix byte, or the u64 slot of a 4-byte remainder, which fits in them; 8 for a record).  exchange_buffers: the
+// buffers of a batch, then whether B can grow to hold one.  It must come after every other allocation of the
+// preparation: B grows later, after a collective, where a rank that failed alone would leave the others waiting.
+void exchange_batch(apgk_group* g, int i, FreqMeta& m, uint64_t payload_bytes) {
   apgk_ctx* c = g->rs[i].c;
   uint64_t budget = c->budget_bytes;
   if (const char* e = getenv("APGK_BUDGET_BYTES")) { if (atoll(e) > 0) budget = (uint64_t)atoll(e); }   // tests: a small device
-  m.batch_bases = std::min<uint64_t>(std::max<uint64_t>(budget / (c->elem_bytes + 4), 4096), 1ull << 31) & ~15ull;
+  m.batch_bases = std::min<uint64_t>(std::max<uint64_t>(budget / (c->elem_bytes + payload_bytes), 4096), 1ull << 31) & ~15ull;
 }
 
-int exchange_buffers(apgk_group* g, int i, bool aff, FreqMeta& m) {
+int exchange_buffers(apgk_group* g, int i, Payload pl, FreqMeta& m) {
   RankState& r = g->rs[i];
   apgk_ctx* c = r.c;
   const int me = g->rank0 + i;
@@ -895,7 +905,7 @@ int exchange_buffers(apgk_group* g, int i, bool aff, FreqMeta& m) {
   GCU(c->blocksum.ensure((((size_t)nb + 1 + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * 8));   // what scan_u32 takes
   for (cudaEvent_t& e : r.gev) if (!e) GCU(cudaEventCreate(&e));
   // B grows later, in refresh_exports (peers may have it mapped): here only whether it can
-  const uint64_t need_B = exchange_B_bytes(per, c->elem_bytes, aff);
+  const uint64_t need_B = exchange_B_bytes(per, c->elem_bytes, pl);
   if (need_B > c->B.cap) {
     size_t fr = 0, tot = 0;
     GCU(cudaMemGetInfo(&fr, &tot));
@@ -926,13 +936,13 @@ int gfreq_prepare(apgk_group* g, int i, uint32_t* const* d_out, const uint64_t* 
   if (n_bases[i] && !d_out[i]) GFAIL(APGK_E_ARG, "rank %d: no output buffer", me);
   m.n_bases = n_bases[i];
   GCU(cudaSetDevice(c->device));
-  exchange_batch(g, i, m);
+  exchange_batch(g, i, m, 4);
   GCU(r.gpos.ensure(std::max<uint64_t>(std::min(m.batch_bases, m.n_bases), 1) * 4));
-  return exchange_buffers(g, i, false, m);
+  return exchange_buffers(g, i, PL_FREQ, m);
 }
 
-// The batch loop both exchanges over the ranks' read stores run (the lookups and the affix build; the kernels are
-// described in gfreq.cuh and gaffix.cuh).  Every rank's B is grown and re-exported to hold one batch (need_B(s) bytes
+// The batch loop the exchanges over the ranks' read stores run (the lookups, the affix and the occurrence builds; the
+// kernels are described in gfreq.cuh, gaffix.cuh and gocc.cuh).  Every rank's B is grown and re-exported to hold one batch (need_B(s) bytes
 // for rank s), then, per batch of BB bases of every local rank's range [first_base[i], + meta.n_bases):
 //   sender  the batch's windows counted by coarse bucket into sizes32 (k_occ_scatter), scanned into the rank's own
 //           piece offsets and the bucket cursors; place(i, b0, first, nbb, tp, grid) puts the elements into B
@@ -1076,7 +1086,7 @@ int group_read_freqs_typed(apgk_group* g, uint32_t* const* d_out, const uint64_t
   constexpr int NT = 128;
   uint64_t BB, n_batches;
   exchange_plan(meta, BB, n_batches);
-  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, false); };
+  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, PL_FREQ); };
   auto start = [&](int) { return APGK_OK; };
   // sender: every window's element into B bucket-major, its batch-relative position at the same slot of gpos
   auto place = [&](int i, uint64_t b0, uint64_t first, uint64_t nbb, const FreqTable<W>& tp, unsigned grid) -> int {
@@ -1178,9 +1188,9 @@ int gaff_prepare(apgk_group* g, int i, FreqMeta& m) {
     GFAIL(APGK_E_STATE, "rank %d: its context was reset, given reads or counted on its own since apgk_group_count: count again", me);
   m.n_bases = c->total_bases;
   GCU(cudaSetDevice(c->device));
-  exchange_batch(g, i, m);
+  exchange_batch(g, i, m, 4);
   GCU(c->aff.ensure(((c->n_distinct + 3) & ~3ull) + 4));
-  return exchange_buffers(g, i, true, m);
+  return exchange_buffers(g, i, PL_AFF, m);
 }
 
 template <int W, typename Elem>
@@ -1193,8 +1203,8 @@ int group_build_affixes_typed(apgk_group* g, const std::vector<FreqMeta>& meta, 
   exchange_plan(meta, BB, n_batches);
   // the byte planes' offsets in the senders' B follow from the all-gathered sizes: every owner knows them unasked
   std::vector<uint64_t> plane(world), first_base(g->n_local, 0);
-  for (int s = 0; s < world; s++) plane[s] = aff_plane(std::min(BB, meta[s].n_bases), eb);
-  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, true); };
+  for (int s = 0; s < world; s++) plane[s] = payload_plane(std::min(BB, meta[s].n_bases), eb, PL_AFF);
+  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, PL_AFF); };
   for (RankState& r : g->rs) { r.c->have_aff = false; r.c->aff_group = false; }
   // the plane offsets beside the peers' pointers; the affix array zeroed (timed with the call: part of its cost)
   auto start = [&](int i) -> int {
@@ -1284,6 +1294,207 @@ int group_build_affixes(apgk_group* g, apgk_group_affix_stats* st) {
   if (c0->W == 1) return group_build_affixes_typed<1, Key<1>>(g, meta, st);
   if (c0->W == 2) return group_build_affixes_typed<2, Key<2>>(g, meta, st);
   return group_build_affixes_typed<3, Key<3>>(g, meta, st);
+}
+
+
+// ---------------------------------------------------------------- occurrence records on the sharded table
+// apgk_group_build_occurrences; the kernels and the data flow are described in gocc.cuh.
+
+int gocc_prepare(apgk_group* g, int i, FreqMeta& m) {
+  RankState& r = g->rs[i];
+  apgk_ctx* c = r.c;
+  const int me = g->rank0 + i;
+  m = FreqMeta{};
+  m.cap_B = c->B.cap; m.cap_sub = c->sub_sizes.cap;
+  m.ptr_B = (uint64_t)(uintptr_t)c->B.p; m.ptr_sub = (uint64_t)(uintptr_t)c->sub_sizes.p;
+  if (!g->counted || !g->freq_ready)
+    GFAIL(APGK_E_STATE, "apgk_group_build_occurrences needs a completed apgk_group_count with APGK_WANT_COUNTS");
+  if (c->gen != r.gen_counted)
+    GFAIL(APGK_E_STATE, "rank %d: its context was reset, given reads or counted on its own since apgk_group_count: count again", me);
+  if (c->max_read_len > (1ull << 31))
+    GFAIL(APGK_E_RANGE, "rank %d: a read of %llu bases (a record keeps the position in a read in 31 bits)", me,
+          (unsigned long long)c->max_read_len);
+  m.n_bases = c->total_bases; m.n_reads = c->n_reads;
+  GCU(cudaSetDevice(c->device));
+  GCTX(c, wait_ingest(c));
+  c->have_occ = false; c->occ_group = false; c->n_occ = 0; c->n_big_runs = 0;   // the buffers below may move
+  // the records take the room of the count's temp buffers, dead until the next count (the shard table is elsewhere):
+  // at 8 B per instance they would not fit beside them at the sizes the group exists for
+  for (DevBuf* b : {&c->A, &c->T, &c->C2, &c->TK}) b->release();
+  c->part_ready = false; c->part_n = 0; c->tmp_keys_last = nullptr;
+  const uint64_t N = c->n_instances, D = c->n_distinct;
+  if (D) GCTX(c, occ_run_offsets(c));   // APGK_E_RANGE when a count saturated
+  else { GCU(c->occ_off.ensure(8)); GCU(cudaMemsetAsync(c->occ_off.p, 0, 8, c->stream)); }
+  GCU(c->occ.ensure(std::max<uint64_t>(N, 1) * 8));
+  GCU(c->occ_cur.ensure(std::max<uint64_t>(D, 1) * 4));
+  GCU(c->occ_big.ensure((N / OCC_SMALL_MAX + 1) * 8));   // a run above OCC_SMALL_MAX takes at least that many slots
+  GCU(c->occ_cnt.ensure(64));
+  for (cudaEvent_t& e : c->occ_ev) if (!e) GCU(cudaEventCreate(&e));
+  // rank directory over the start bitmap: the sweep numbers the reads of this store (a store without bases has no
+  // bitmap, and no window to number)
+  if (c->total_bases) {
+    const uint64_t words = (c->total_bases + 31) / 32;
+    const uint64_t n_blocks = words / RANK_BLOCK_WORDS + 1;   // covers word index `words` as well; the bitmap is zero padded
+    GCU(c->rank_cnt.ensure(n_blocks * 4));
+    GCU(c->rank_dir.ensure((n_blocks + 1) * 8));
+    k_start_blocks<<<(unsigned)((n_blocks + 255) / 256), 256, 0, c->stream>>>(c->starts.as<uint32_t>(), n_blocks, c->rank_cnt.as<uint32_t>());
+    c->launches++;
+    GCU(cudaGetLastError());
+    GCTX(c, scan_u32(c, c->rank_cnt.as<uint32_t>(), n_blocks, c->rank_dir.as<unsigned long long>(), nullptr));
+  }
+  if (!c->empty_nb.empty()) {
+    GCU(c->empty_dev.ensure(c->empty_nb.size() * 8));
+    GCU(cudaMemcpyAsync(c->empty_dev.p, c->empty_nb.data(), c->empty_nb.size() * 8, cudaMemcpyHostToDevice, c->stream));
+  }
+  exchange_batch(g, i, m, 8);
+  return exchange_buffers(g, i, PL_OCC, m);
+}
+
+template <int W, typename Elem>
+int group_build_occurrences_typed(apgk_group* g, const std::vector<FreqMeta>& meta, const std::vector<uint64_t>& read_base,
+                                  apgk_group_occ_stats* st) {
+  const int world = g->world, nl = g->n_local;
+  constexpr uint64_t eb = sizeof(Elem);
+  constexpr int NT = 128;
+  uint64_t BB, n_batches;
+  exchange_plan(meta, BB, n_batches);
+  // the record planes' offsets in the senders' B follow from the all-gathered sizes: every owner knows them unasked
+  std::vector<uint64_t> plane(world), first_base(nl, 0);
+  for (int s = 0; s < world; s++) plane[s] = payload_plane(std::min(BB, meta[s].n_bases), eb, PL_OCC);
+  auto need_B = [&](int s) { return exchange_B_bytes(std::min(BB, meta[s].n_bases), eb, PL_OCC); };
+  // the plane offsets beside the peers' pointers; the run cursors zeroed (timed with the call: part of its cost)
+  auto start = [&](int i) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    GCU(cudaMemcpyAsync(r.ptrs_dev.as<unsigned char>() + (size_t)world * 8, plane.data(), (size_t)world * 8, cudaMemcpyHostToDevice, c->stream));
+    GCU(cudaMemsetAsync(c->occ_cur.p, 0, std::max<uint64_t>(c->n_distinct, 1) * 4, c->stream));
+    return APGK_OK;
+  };
+  // sender: every window's element and record into B bucket-major; counters[3] += the windows placed
+  auto place = [&](int i, uint64_t, uint64_t first, uint64_t nbb, const FreqTable<W>& tp, unsigned grid) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    const int me = g->rank0 + i;
+    unsigned long long* cnt = r.gcnt.as<unsigned long long>();
+    GoccReads rd{c->rank_dir.as<unsigned long long>(), c->empty_dev.as<unsigned long long>(), (uint32_t)c->empty_nb.size(), read_base[me]};
+    k_gocc_scatter<W, Elem, NT><<<grid, NT, 0, c->stream>>>(read_store(c), tp, first, nbb, c->occ_bcur.as<unsigned long long>(), c->B.as<Elem>(),
+                                                           reinterpret_cast<unsigned long long*>(c->B.as<uint8_t>() + plane[me]), nbb, rd, cnt);
+    c->launches++;
+    GCU(cudaGetLastError());
+    k_gaff_sent<<<1, 1, 0, c->stream>>>(c->piece_off.as<unsigned long long>() + (size_t)me * ((size_t)r.nb + 1) + r.nb, cnt);
+    c->launches++;
+    GCU(cudaGetLastError());
+    return APGK_OK;
+  };
+  // owner: the pieces of its buckets read from the senders' B, every record stored into its own run
+  auto own = [&](int i, const FreqTable<W>& ts) -> int {
+    RankState& r = g->rs[i];
+    apgk_ctx* c = r.c;
+    const int me = g->rank0 + i;
+    GoccArgs a{};
+    a.src = (const void* const*)r.ptrs_dev.p;
+    a.plane_off = r.ptrs_dev.as<unsigned long long>() + world;
+    a.piece_off = c->piece_off.as<unsigned long long>();
+    a.n_src = (uint32_t)world; a.nb = r.nb; a.me = (uint32_t)me;
+    a.d2 = r.geom_shard.D1 - r.geom_part.D1; a.rem_bits = r.geom_part.REM; a.pad = r.geom_part.pad;
+    a.run_off = c->occ_off.as<unsigned long long>();
+    a.cursor = c->occ_cur.as<uint32_t>();
+    a.occ = c->occ.as<unsigned long long>();
+    a.counters = r.gcnt.as<unsigned long long>();
+    for (const auto& sg : g->own_segs) {
+      if ((int)sg[2] != me) continue;
+      a.lo = sg[0]; a.hi = sg[1];
+      k_gocc_place<W, Elem, OCC_PLACE_NT><<<std::min<uint32_t>(sg[1] - sg[0], (uint32_t)c->n_sm * 8), OCC_PLACE_NT, 0, c->stream>>>(ts, a);
+      c->launches++;
+      GCU(cudaGetLastError());
+    }
+    return APGK_OK;
+  };
+  auto after = [&](int, uint64_t, uint64_t) { return APGK_OK; };   // nothing comes back to the sender
+  unsigned long long red[4] = {0, 0, 0, 0}, cnt[4] = {0, 0, 0, 0};
+  float ms[3], total = 0;
+  { int rc = exchange_batches<W, Elem>(g, meta, first_base.data(), BB, n_batches, need_B, start, place, own, after, red, cnt, ms, &total); if (rc) return rc; }
+  if (red[0] || red[2])
+    GFAIL(APGK_E_STATE, "group occurrences: %llu windows missing from their owner's table, %llu beyond their bucket or run (the tables do not match the reads)",
+          red[0], red[2]);
+  // every run ascending: the runs filled piece by piece, batch after batch, so they arrive as several sorted sequences
+  std::vector<unsigned long long> n_big(nl, 0);
+  for (int i = 0; i < nl; i++) {
+    apgk_ctx* c = g->rs[i].c;
+    const uint64_t D = c->n_distinct;
+    GCU(cudaSetDevice(c->device));
+    unsigned long long* sc = c->occ_cnt.as<unsigned long long>();
+    GCU(cudaMemsetAsync(sc, 0, 32, c->stream));
+    GCU(cudaEventRecord(c->occ_ev[3], c->stream));
+    if (D) {
+      k_occ_sort_small<<<(unsigned)((D + 127) / 128), 128, 0, c->stream>>>(c->occ_off.as<unsigned long long>(), D, c->occ.as<unsigned long long>(),
+                                                                          c->occ_big.as<unsigned long long>(), sc);
+      c->launches++;
+      GCU(cudaGetLastError());
+    }
+    GCU(cudaEventRecord(c->occ_ev[4], c->stream));
+    if (D) {
+      k_occ_sort_big<OCC_BIG_NT><<<c->n_sm * 2, OCC_BIG_NT, 0, c->stream>>>(c->occ_off.as<unsigned long long>(), c->occ_big.as<unsigned long long>(),
+                                                                           sc, c->occ.as<unsigned long long>());
+      c->launches++;
+      GCU(cudaGetLastError());
+    }
+    GCU(cudaEventRecord(c->occ_ev[5], c->stream));
+    GCU(cudaMemcpyAsync(&n_big[i], sc, 8, cudaMemcpyDeviceToHost, c->stream));
+  }
+  for (int i = 0; i < nl; i++) {
+    apgk_ctx* c = g->rs[i].c;
+    GCU(cudaSetDevice(c->device));
+    GCU(cudaStreamSynchronize(c->stream));
+    for (float& x : c->occ_ms) x = 0;
+    if (i == 0) { c->occ_ms[1] = ms[0]; c->occ_ms[2] = ms[1]; }
+    cudaEventElapsedTime(&c->occ_ms[3], c->occ_ev[3], c->occ_ev[4]);
+    cudaEventElapsedTime(&c->occ_ms[4], c->occ_ev[4], c->occ_ev[5]);
+    c->n_big_runs = n_big[i];
+    c->n_occ = c->n_instances;
+    c->have_occ = true; c->occ_group = true;
+  }
+  if (st) {
+    apgk_ctx* c0 = g->rs[0].c;
+    *st = apgk_group_occ_stats{};
+    st->n_batches = (int32_t)n_batches;
+    st->n_windows = cnt[3];
+    st->n_occ = c0->n_occ;
+    st->n_big_runs = c0->n_big_runs;
+    st->remote_bytes = cnt[1] * (eb + 8);
+    st->sweep_ms = ms[0]; st->exchange_ms = ms[1];
+    st->sort_ms = c0->occ_ms[3] + c0->occ_ms[4];
+    if (cudaEventElapsedTime(&st->total_ms, g->rs[0].gev[4], c0->occ_ev[5]) != cudaSuccess) st->total_ms = total + st->sort_ms;
+  }
+  return APGK_OK;
+}
+
+int group_build_occurrences(apgk_group* g, apgk_group_occ_stats* st) {
+  if (g->dead) GFAIL(APGK_E_STATE, "a context of this group has been destroyed");
+  const int world = g->world, nl = g->n_local;
+  std::vector<FreqMeta> mine(nl), meta(world);
+  std::string own_err;
+  for (int i = 0; i < nl; i++) {
+    const int rc = gocc_prepare(g, i, mine[i]);
+    if (rc) { mine[i].status = rc; if (own_err.empty()) own_err = g->err; }
+  }
+  { int rc = coll_allgather_host(g, mine.data(), sizeof(FreqMeta), meta.data()); if (rc) return rc; }
+  for (int s = 0; s < world; s++)
+    if (meta[s].status) {
+      if (own_err.empty()) GFAIL(meta[s].status, "rank %d refused the occurrence build (error %d; its apgk_group_last_error says why)", s, meta[s].status);
+      g->err = own_err;
+      return meta[s].status;
+    }
+  // group read ids: every rank's reads in rank order (the same numbers on every rank)
+  std::vector<uint64_t> read_base(world + 1, 0);
+  for (int s = 0; s < world; s++) read_base[s + 1] = read_base[s] + meta[s].n_reads;
+  if (read_base[world] > 0xFFFFFFFFull)
+    GFAIL(APGK_E_RANGE, "group occurrences: read ids are 32-bit, %llu reads in the group", (unsigned long long)read_base[world]);
+  apgk_ctx* c0 = g->rs[0].c;
+  if (c0->elem_bytes == 4) return group_build_occurrences_typed<1, uint32_t>(g, meta, read_base, st);
+  if (c0->W == 1) return group_build_occurrences_typed<1, Key<1>>(g, meta, read_base, st);
+  if (c0->W == 2) return group_build_occurrences_typed<2, Key<2>>(g, meta, read_base, st);
+  return group_build_occurrences_typed<3, Key<3>>(g, meta, read_base, st);
 }
 
 }  // namespace

@@ -24,6 +24,7 @@
 //               CTA-wide bitonic network (shared memory up to OCC_SH_CAP entries, else in place).
 // The result is deterministic (independent of atomic order).  (read id, position) are derived from
 // the global position on demand by k_occ_translate through a rank directory over the start bitmap.
+// (The records of a shard, apgk_group_build_occurrences, are built in read-id form instead: gocc.cuh.)
 #pragma once
 #include "table.cuh"
 
@@ -320,26 +321,26 @@ __global__ void k_start_blocks(const uint32_t* __restrict__ starts32, uint64_t n
   cnt[i] = s;
 }
 
-// occ[i] = (q << 1 | rc) -> read_id[i], pos[i]: pos is 1-based in the read, negative when the canonical
-// form is the reverse complement of the read's window (SortKmers record convention, SURVEY.md 8(a) [U]).
-// Reads without bases own no start bit: empty_nb[e] = non-empty reads before the e-th empty read (ascending)
-// shifts the rank back to the caller's read numbering.
-__global__ void k_occ_translate(const unsigned long long* __restrict__ occ, uint64_t n, const uint32_t* __restrict__ starts32,
-                                const unsigned long long* __restrict__ blk_rank, const unsigned long long* __restrict__ empty_nb,
-                                uint32_t n_empty, uint32_t* __restrict__ read_id, int32_t* __restrict__ pos) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const unsigned long long v = occ[i];
-  const uint64_t q = v >> 1;
+// The read holding global base position q, in two halves (the group build's sweep, gocc.cuh, reuses the first
+// for a thread's first window and derives its other windows from the start bits it already holds):
+// occ_start_rank: rank = read starts at positions <= q (rank directory + popcounts), s = the start of q's read.
+__device__ __forceinline__ void occ_start_rank(const uint32_t* __restrict__ starts32, const unsigned long long* __restrict__ blk_rank,
+                                               uint64_t q, unsigned long long& rank, uint64_t& s) {
   const uint64_t wq = q >> 5, blk = wq / RANK_BLOCK_WORDS;
-  unsigned long long rank = blk_rank[blk];
+  rank = blk_rank[blk];
   for (uint64_t w = blk * RANK_BLOCK_WORDS; w < wq; w++) rank += __popc(starts32[w]);
   uint32_t bits = starts32[wq] & (0xFFFFFFFFu >> (31u - (uint32_t)(q & 31)));  // starts at positions <= q
   rank += __popc(bits);
   uint64_t w = wq;
   while (!bits && w > 0) bits = starts32[--w];
-  const uint64_t s = (w << 5) + (bits ? 31u - (uint32_t)__clz((int)bits) : 0u);  // start of the read holding q
-  unsigned long long id = rank ? rank - 1 : 0;  // rank among the reads that have bases
+  s = (w << 5) + (bits ? 31u - (uint32_t)__clz((int)bits) : 0u);  // start of the read holding q
+}
+
+// occ_read_id: the rank among the reads that have bases -> the caller's read numbering.  Reads without bases own
+// no start bit: empty_nb[e] = non-empty reads before the e-th empty read (ascending) shifts the rank back.
+__device__ __forceinline__ unsigned long long occ_read_id(unsigned long long rank, const unsigned long long* __restrict__ empty_nb,
+                                                          uint32_t n_empty) {
+  unsigned long long id = rank ? rank - 1 : 0;
   if (n_empty) {
     uint32_t lo = 0, hi = n_empty;               // number of empty reads with empty_nb <= id
     while (lo < hi) {
@@ -348,6 +349,22 @@ __global__ void k_occ_translate(const unsigned long long* __restrict__ occ, uint
     }
     id += lo;
   }
+  return id;
+}
+
+// occ[i] = (q << 1 | rc) -> read_id[i], pos[i]: pos is 1-based in the read, negative when the canonical
+// form is the reverse complement of the read's window (SortKmers record convention, SURVEY.md 8(a) [U]).
+__global__ void k_occ_translate(const unsigned long long* __restrict__ occ, uint64_t n, const uint32_t* __restrict__ starts32,
+                                const unsigned long long* __restrict__ blk_rank, const unsigned long long* __restrict__ empty_nb,
+                                uint32_t n_empty, uint32_t* __restrict__ read_id, int32_t* __restrict__ pos) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const unsigned long long v = occ[i];
+  const uint64_t q = v >> 1;
+  unsigned long long rank;
+  uint64_t s;
+  occ_start_rank(starts32, blk_rank, q, rank, s);
+  const unsigned long long id = occ_read_id(rank, empty_nb, n_empty);
   const int32_t p1 = (int32_t)(q - s) + 1;
   read_id[i] = (uint32_t)id;
   pos[i] = (v & 1ull) ? -p1 : p1;

@@ -106,6 +106,18 @@ def sharded_affixes(kc, rank, world, group=None, stats=None):
     return kc.affixes()
 
 
+def sharded_occurrences(kc, rank, world, group=None, stats=None):
+    """After `sharded_count`: the occurrence records of every row of this rank's shard table (the rows of
+    `kc.counts()`), taken over ALL ranks' reads, as host arrays (run_off, read_id, pos) like kc.occurrences().  Read
+    ids are group read ids: rank 0's reads first, then each rank's in order.  Collective: every rank calls it
+    (apgk_group_build_occurrences).  The records stay in `kc` for kc.occurrences() / kc.occurrences_device()."""
+    grp = _group_of(kc, rank, world, group)
+    st = grp.build_occurrences()
+    if stats is not None:
+        stats.update(st)
+    return kc.occurrences()
+
+
 def _group_of(kc, rank, world, group=None):
     """The library-side group of this counter (made once: rank 0's id is broadcast over torch.distributed)."""
     from .kmers import KmerGroup

@@ -212,7 +212,8 @@ class KmerCounter:
     def occurrences(self, first=0, n=None):
         """-> (run_off uint64[n+1] rebased to 0, read_id uint32[m], pos int32[m]) for k-mers [first, first+n) of
         the sorted table; k-mer first+i owns slots [run_off[i], run_off[i+1]), ascending by (read id, position);
-        pos is 1-based, negative when the canonical form is the reverse complement of the read's window."""
+        pos is 1-based, negative when the canonical form is the reverse complement of the read's window.  On a shard
+        after KmerGroup.build_occurrences() the read ids are group read ids."""
         _, nd = self.totals()
         if n is None:
             n = nd - first
@@ -226,6 +227,8 @@ class KmerCounter:
         return ro - ro[0], rid[:m], pos[:m]
 
     def occurrences_device(self):
+        """-> (device pointer of the run offsets, device pointer of the records, n_occ); the record encoding is
+        include/apgk.h's (read-id form on a shard after KmerGroup.build_occurrences())."""
         a, b = C.c_void_p(), C.c_void_p()
         n = C.c_uint64()
         self._ck(self._L.apgk_occurrences_device(self._h, C.byref(a), C.byref(b), C.byref(n)))
@@ -492,6 +495,15 @@ class KmerGroup:
         -> dict(n_batches, n_windows, remote_bytes, sweep_ms, exchange_ms, total_ms)."""
         st = _lib.GroupAffixStats()
         self._ck(self._L.apgk_group_build_affixes(self._h, C.byref(st)))
+        return {k: getattr(st, k) for k, _ in st._fields_}
+
+    def build_occurrences(self):
+        """K-mer occurrence records on the sharded table (collective): afterwards every local counter's occurrences() /
+        occurrences_device() answer for the rows of its shard, taken over all ranks' reads, with GROUP read ids (every
+        rank's reads in rank order).  -> dict(n_batches, n_windows, n_occ, n_big_runs, remote_bytes, sweep_ms,
+        exchange_ms, sort_ms, total_ms)."""
+        st = _lib.GroupOccStats()
+        self._ck(self._L.apgk_group_build_occurrences(self._h, C.byref(st)))
         return {k: getattr(st, k) for k, _ in st._fields_}
 
     def _ranges(self, first_base, n_bases):

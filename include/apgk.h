@@ -171,7 +171,10 @@ int apgk_build_occurrences(apgk_ctx* ctx);
  * placement, per-run sort, big-run sort}. */
 int apgk_occurrences_info(const apgk_ctx* ctx, uint64_t* n_occ, uint64_t* n_big_runs, float* ms5);
 /* DEVICE pointers, library-owned until the next finish / reset: run offsets (uint64[n_distinct+1]) and
- * the occurrences encoded as (global base position in the read store << 1) | canonical_is_reverse. */
+ * the occurrences encoded as (global base position in the read store << 1) | canonical_is_reverse.
+ * On a shard whose records come from apgk_group_build_occurrences the encoding is different: the sender has already
+ * numbered the read, so a record is (group read id << 32) | ((position in read - 1) << 1) | canonical_is_reverse.
+ * Its ascending u64 order is ascending (read id, position), as in the single-GPU encoding. */
 int apgk_occurrences_device(apgk_ctx* ctx, const uint64_t** d_run_off, const uint64_t** d_occ, uint64_t* n_occ);
 /* HOST copies for k-mers [first_kmer, first_kmer + n_kmers): run_off_out[n_kmers+1] (absolute slots; may
  * be NULL), and read_id_out / pos_out for slots [run_off[first_kmer], run_off[first_kmer+n_kmers)) (both
@@ -376,6 +379,35 @@ typedef struct {
   float sweep_ms, exchange_ms, total_ms;   /* device time, first local context */
 } apgk_group_affix_stats;
 int apgk_group_build_affixes(apgk_group* g, apgk_group_affix_stats* stats);
+/* K-mer occurrence records on the sharded table: apgk_build_occurrences for a group.  After apgk_group_count with
+ * APGK_WANT_COUNTS, every local context holds the records of the rows of its shard table, taken over ALL ranks' reads:
+ * run_off is the exclusive scan of the shard's counts, each run is ascending by (read id, position), pos is 1-based and
+ * negative when the canonical form is the reverse complement (a palindrome counts as forward).  Read ids are GROUP
+ * read ids: the reads of every rank in rank order (rank 0's first; in the single-process form, the order of the
+ * contexts given to apgk_group_local), each rank's in the order they were added, reads without bases included.  So a
+ * group's records equal what apgk_build_occurrences gives on one context holding all ranks' reads back to back.
+ * Every window's level-1 element and record travel to the k-mer's owner on the query exchange of
+ * apgk_group_read_freqs_device (per batch of the rank's whole read store; every rank runs the same number of batches);
+ * the owner reads the pieces of its buckets over peer memory and stores each record into its own run.  Nothing is
+ * written to a peer.  Afterwards apgk_occurrences_info / apgk_occurrences_device (read-id encoding, see above) /
+ * apgk_occurrences_copy answer on each shard; info's ms5 are {0, sweep, exchange, per-run sort, big-run sort}, the
+ * first two on the group's first local context only.  The records survive apgk_group_read_freqs_device and
+ * apgk_group_build_affixes; they are dropped by apgk_release_temp (as on one GPU) and by whatever drops the shard
+ * table.  apgk_build_occurrences on a shard still refuses with APGK_E_STATE.
+ * Collective; stats may be NULL.  Errors come back identical on every rank: APGK_E_STATE without a current count with
+ * APGK_WANT_COUNTS, when a member context was reset, given reads or counted on its own since (apgk_release_temp is
+ * fine), or when a window's k-mer is missing from its owner's table (the records are then not built on any rank);
+ * APGK_E_RANGE for more than 2^32 - 1 group reads, a read longer than 2^31 bases or a shard count that saturated;
+ * APGK_E_NOMEM when a rank's records, run offsets, cursors and batch buffers do not fit. */
+typedef struct {
+  int32_t n_batches;      /* exchange batches this call ran (agreed by all ranks) */
+  uint64_t n_windows;     /* valid windows of this rank's read store that were sent */
+  uint64_t n_occ;         /* records of this rank's shard (== its apgk_totals n_instances) */
+  uint64_t n_big_runs;    /* runs of this shard sorted by the CTA-wide network */
+  uint64_t remote_bytes;  /* bytes this rank's owner-side kernel read from peers' memory */
+  float sweep_ms, exchange_ms, sort_ms, total_ms;   /* device time, first local context */
+} apgk_group_occ_stats;
+int apgk_group_build_occurrences(apgk_group* g, apgk_group_occ_stats* stats);
 
 /* ---- instrumentation */
 #define APGK_N_STAGES 14
