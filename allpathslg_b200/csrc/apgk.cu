@@ -984,14 +984,24 @@ int count_buckets(apgk_ctx* c, uint64_t Nr, uint64_t N, uint64_t& n_prev, Key<W>
     CU(cudaMemsetAsync(c->deferred.p, 0, 4, c->stream));
     stage_begin(c, ST_LOCAL);
     if (use_l3) {
-      // 32-bit remainders: order-preserving hash kernel; it takes every bucket size (range splitting)
+      // 32-bit remainders: a small CTA per bucket with a table for its distinct keys; buckets it cannot take land
+      // on the deferred list ...
       if constexpr (std::is_same<ElemB, uint32_t>::value) {
+        auto kern5 = k_local5<W>;
+        int occ5 = 1;
+        { int rc = kernel_setup(c, kern5, L5_NT, L5_SMEM, &occ5); if (rc) return rc; }
+        const uint32_t grid5 = std::max<uint32_t>(1, std::min<uint32_t>(bt.nb - bt.b0, (uint32_t)(c->n_sm * std::max(occ5, 1))));
+        kern5<<<grid5, L5_NT, L5_SMEM, c->stream>>>((const uint32_t*)c->count_src, bt, g.REM, ec, c->nd.as<uint32_t>(),
+                                                     c->deferred.as<uint32_t>(), c->nb1);
+        LAUNCHED();
+        // ... which the order-preserving kernel then walks: it takes every bucket size (range splitting)
         auto launch3 = [&](auto kern3, int nt) -> int {
           const size_t sm3 = Local3Smem::bytes(local_max);
           int occ3 = 1;
           { int rc = kernel_setup(c, kern3, nt, sm3, &occ3); if (rc) return rc; }
           const uint32_t grid3 = std::min<uint32_t>(c->nb1, (uint32_t)(c->n_sm * std::max(occ3, 1)));
-          kern3<<<grid3, nt, sm3, c->stream>>>((const uint32_t*)c->count_src, bt, g.REM, ec, c->nd.as<uint32_t>());
+          kern3<<<grid3, nt, sm3, c->stream>>>((const uint32_t*)c->count_src, bt, g.REM, ec, c->nd.as<uint32_t>(),
+                                               c->deferred.as<uint32_t>(), c->nb1);
           return APGK_OK;
         };
         int rc3 = l3_nt == 256 ? launch3(k_local3<256, W>, 256) : launch3(k_local3<512, W>, 512);

@@ -1,5 +1,8 @@
 // local3.cuh -- sort-and-count for 32-bit remainders by ORDER-PRESERVING hashing.
 //
+// It walks the buckets k_local5 (local5.cuh) defers: those with more distinct keys than k_local5's table or more
+// instances than its 16-bit counts.  It takes every bucket size, so it is the fallback.
+//
 // Keys of one bucket share their leading bits, so the remainder r (< 2^REM) of a
 // random-looking genome is spread evenly.  The table is cut into ROWS of 16 slots and
 // the row of a key is chosen MONOTONE in the key:   row(r) = floor(r * nrows / 2^REM);
@@ -78,9 +81,11 @@ struct Local3Smem {
   }
 };
 
+// Buckets list[1 .. 1 + min(list[0], list_cap)).
 template <int NT, int W>
 __global__ void __launch_bounds__(NT, 1536 / NT) k_local3(const uint32_t* __restrict__ src, BucketTable bt, int rem_bits, EmitCtx<W> ec,
-                                               uint32_t* __restrict__ nd_out) {
+                                               uint32_t* __restrict__ nd_out, const uint32_t* __restrict__ list,
+                                               uint32_t list_cap) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Local3Smem sm;
   const int LM = (int)bt.local_max;
@@ -93,14 +98,17 @@ __global__ void __launch_bounds__(NT, 1536 / NT) k_local3(const uint32_t* __rest
   // The next bucket's size / offset are loaded one bucket ahead and its keys are pulled toward L2 while
   // the current bucket is processed: a CTA otherwise sits through two dependent DRAM latencies per
   // bucket (bsize/bofs, then the keys) and three CTAs per SM do not cover them.
+  const uint32_t n_iter = list[0] < list_cap ? list[0] : list_cap;
+  uint32_t b_nx = 0;
   unsigned long long n_nx = 0, o_nx = 0;
-  if (bt.b0 + blockIdx.x < bt.nb) { n_nx = bt.bsize[bt.b0 + blockIdx.x]; o_nx = bt.bofs[bt.b0 + blockIdx.x]; }
-  for (uint32_t b = bt.b0 + blockIdx.x; b < bt.nb; b += gridDim.x) {
+  if (blockIdx.x < n_iter) { b_nx = list[1 + blockIdx.x]; n_nx = bt.bsize[b_nx]; o_nx = bt.bofs[b_nx]; }
+  for (uint32_t it = blockIdx.x; it < n_iter; it += gridDim.x) {
+    const uint32_t b = b_nx;
     const unsigned long long n64 = n_nx;
     const unsigned long long o = o_nx;
     {
-      const uint32_t bn = b + gridDim.x;
-      if (bn < bt.nb) { n_nx = bt.bsize[bn]; o_nx = bt.bofs[bn]; }
+      const uint32_t itn = it + gridDim.x;
+      if (itn < n_iter) { b_nx = list[1 + itn]; n_nx = bt.bsize[b_nx]; o_nx = bt.bofs[b_nx]; }
     }
     if (n64 == 0) {
       if (tid == 0) nd_out[b] = 0;
@@ -180,7 +188,7 @@ __global__ void __launch_bounds__(NT, 1536 / NT) k_local3(const uint32_t* __rest
 #if L3_PREFETCH
       if (L3_PREFETCH == 1 || run_nd == 0) {  // next bucket's keys toward L2 (32 keys per 128-byte line)
         const unsigned long long i = (unsigned long long)tid * 32;
-        if (b + gridDim.x < bt.nb && i < n_nx && tid < 1024) prefetch_l2(src + o_nx + i);
+        if (it + gridDim.x < n_iter && i < n_nx && tid < 1024) prefetch_l2(src + o_nx + i);
       }
 #endif
       // ---- 3. dense list of occupied slots, in slot order

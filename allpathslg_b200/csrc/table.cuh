@@ -4,6 +4,7 @@
 // BASELINE.json north_star; SURVEY.md section 3.2 -- no file:line available).
 #pragma once
 #include "local4.cuh"
+#include "local5.cuh"
 
 namespace apgk {
 
